@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload wg|c1|st] [--d-model 128|512] [--variant base|layers3|gateoff|normnone|hic1000000|hic125000]
-                    [--rounds R]
+                    [--rounds R] [--dump-outputs DIR]
 
 Metric (BASELINE.json): "GCN train step edges/sec (GE/s)".  A step is one pass of the hot path over the workload: for
 every chromosome graph, both strands through the gated GCN, BCE loss, backward, optimiser step (finetune.py:29-49).
@@ -75,7 +75,56 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--gemm-impl", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (probabilities of a fixed row sample, "
+                         "losses, model state) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path; the reference arm has nothing to dump")
+    return args
+
+
+DUMP_PROB_BYTES = 32 << 20       # probabilities --dump-outputs writes per run, spread over the workload's graphs
+
+
+def dump_rows(n, n_graphs, seed):
+    """Sorted row indices of the fixed sample of an n-row probability matrix that --dump-outputs writes."""
+    import numpy as np
+    k = max(1, DUMP_PROB_BYTES // (4 * NCLASS * n_graphs))
+    return np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir, torch, arrays):
+    """Write host copies of the given tensors as out_dir/<name>.npy: float64 stays float64, the rest becomes float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy() if t.dtype == torch.float64 else t.float().numpy())
+
+
+def last_step_losses(acc):
+    """--dump-outputs: the loss slots accumulate (`+=`) over every pass.  `before()` runs right before the last timed
+    step and zeroes them; `after()` then returns exactly that step's losses and adds the earlier sum back (one fp32
+    add per slot, so the running sum ends bit-identical to a run without the dump)."""
+    prior = []
+
+    def before():
+        prior.append(acc.clone())
+        acc.zero_()
+
+    def after():
+        last = acc.clone()
+        acc.add_(prior[0])
+        return last
+    return before, after
+
+
+def dump_model_state(out_dir, torch, model):
+    dump_outputs(out_dir, torch, {"model." + k: v.double() if v.dtype == torch.int64 else v
+                                  for k, v in model.state_dict().items()})
 
 
 def variant_cfg(args):
@@ -178,7 +227,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(args.steps, 1)
+    steps = args.steps
     chroms = ["chr22"] if args.workload == "c1" else (CPU_SAMPLE if args.workload == "st" else workload_chroms("wg"))
     budget = float(os.environ.get("CGCN_REF_BUDGET_S", "900"))
     same_config = args.workload != "st"
@@ -411,7 +460,7 @@ def run_chromosomes(args, torch, dist, dev, world, rank, sampler):
     from chromegcn_b200.engine import ChromosomeEngine
     from chromegcn_b200.graph import HiCGraph
     from chromegcn_b200.optim import FlatSGD
-    steps, warmup = max(args.steps, 1), max(args.warmup, 3)
+    steps, warmup = args.steps, max(args.warmup, 3)
     layers, gate, extended, hic, use_norm = variant_cfg(args)
     D = args.d
     chroms = workload_chroms(args.workload)
@@ -459,9 +508,23 @@ def run_chromosomes(args, torch, dist, dev, world, rank, sampler):
             dist.barrier()
         torch.cuda.synchronize(dev)
 
-    ms_per_step, launches = timed_region(torch, dist, dev, world, sampler, one_step, barrier, steps, warmup, _lib)
+    before_last, after_last = last_step_losses(losses)
+    ms_per_step, launches = timed_region(torch, dist, dev, world, sampler, one_step, barrier, steps, warmup, _lib,
+                                         before_last if args.dump_outputs else None)
     value = total_edges / (ms_per_step * 1e-3) / 1e9
+    last_losses = after_last() if args.dump_outputs else None
     final_loss = float(losses.sum().item())
+    if args.dump_outputs:
+        # before the e2e passes below train the model further; each rank writes its own chromosomes
+        order = [c for rnd in schedule for c in rnd[rank]]          # losses[i] belongs to order[i]
+        out = {}
+        for i, c in enumerate(order):
+            rows = torch.from_numpy(dump_rows(graphs[c].n, len(chroms), synthetic.chrom_index(c))).to(dev)
+            out["probs." + c] = probs[c].index_select(0, rows)
+            out["loss." + c] = last_losses[i: i + 1]
+        dump_outputs(args.dump_outputs, torch, out)
+        if rank == 0:
+            dump_model_state(args.dump_outputs, torch, model)
 
     # ---- e2e: drop-in finetune() with pinned host features, H2D/D2H inside the timed region, the same rounds at N > 1
     e2e = None
@@ -526,7 +589,7 @@ def run_chromosomes(args, torch, dist, dev, world, rank, sampler):
     return value, ms_per_step, launches, e2e, roofline, config, "strong"
 
 
-def timed_region(torch, dist, dev, world, sampler, one_step, barrier, steps, warmup, _lib):
+def timed_region(torch, dist, dev, world, sampler, one_step, barrier, steps, warmup, _lib, before_last=None):
     sampler.load0 = time.monotonic()
     for _ in range(warmup):
         one_step()
@@ -537,7 +600,9 @@ def timed_region(torch, dist, dev, world, sampler, one_step, barrier, steps, war
     sampler.mark_begin()
     ev0.record()
     torch.cuda.nvtx.range_push("timed")
-    for _ in range(steps):
+    for i in range(steps):
+        if before_last is not None and i == steps - 1:
+            before_last()
         one_step()
     torch.cuda.nvtx.range_pop()
     ev1.record()
@@ -561,7 +626,7 @@ def run_stress(args, torch, dist, dev, world, rank, sampler):
     from chromegcn_b200.chrome_models import ChromeGCN
     from chromegcn_b200.graph import HiCGraph
     from chromegcn_b200.optim import FlatSGD
-    steps, warmup = max(args.steps, 1), max(args.warmup, 3)
+    steps, warmup = args.steps, max(args.warmup, 3)
     D, n = args.d, args.st_rows
     a = synthetic.make_pattern_direct(n, args.st_pairs, seed=77)
     a = (a + sparse.eye(n, format="csr")).tocsr()
@@ -597,8 +662,20 @@ def run_stress(args, torch, dist, dev, world, rank, sampler):
             dist.barrier()
         torch.cuda.synchronize(dev)
 
-    ms_per_step, launches = timed_region(torch, dist, dev, world, sampler, one_step, barrier, steps, warmup, _lib)
+    before_last, after_last = last_step_losses(loss)
+    ms_per_step, launches = timed_region(torch, dist, dev, world, sampler, one_step, barrier, steps, warmup, _lib,
+                                         before_last if args.dump_outputs else None)
     value = total_edges / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs:
+        # before the e2e steps below; the loss and the model state are the same on every rank, the probability budget
+        # is split over the ranks' row blocks
+        last_loss = after_last()
+        name = "probs.st" if world == 1 else "probs.st.rank%d" % rank
+        rows = torch.from_numpy(dump_rows(e - b, world, rank)).to(dev)
+        dump_outputs(args.dump_outputs, torch, {name: probs.index_select(0, rows)})
+        if rank == 0:
+            dump_outputs(args.dump_outputs, torch, {"loss.st": last_loss})
+            dump_model_state(args.dump_outputs, torch, model)
 
     e2e = None
     if not args.no_e2e:
@@ -697,7 +774,7 @@ def main():
                         "sample": "10 train steps on the chr22-sized graph (N=20000, %d stored entries), %.3f s/step; "
                                   "oracle port of the reference PyTorch CPU path incl. host process_graph" % (e_cpu, dt_cpu)}
     if rank == 0:
-        line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": max(args.steps, 1),
+        line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
                 "warmup": max(args.warmup, 3), "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": scaling,
                 "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config, "e2e": e2e,
                 "gpu_launches": launches, "clocks": clocks, "roofline": roofline, "cpu_baseline": cpu_baseline,

@@ -68,6 +68,33 @@ def test_permuted_graph_keeps_degrees_and_symmetry():
     assert not np.array_equal(ix, a.indices)
 
 
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "c1", "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
+def test_dump_row_sample_is_fixed_and_within_budget():
+    """--dump-outputs writes the same rows of every probability matrix on every run and build, 64 MB at most in all:
+    whole-genome graphs share the probability budget, and so do the ranks' row blocks of the st graph."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from chromegcn_b200 import synthetic
+    from chromegcn_b200.dist import row_partition
+    chroms = synthetic.WHOLE_GENOME
+    rows = {c: bench.dump_rows(synthetic.num_windows(c), len(chroms), synthetic.chrom_index(c)) for c in chroms}
+    for c, r in rows.items():
+        assert np.all(np.diff(r) > 0) and 0 <= r[0] and r[-1] < synthetic.num_windows(c)
+    assert rows["chr1"][:4].tolist() == [9, 97, 111, 197] and rows["chr22"][:4].tolist() == [2, 13, 14, 28]
+    assert sum(r.size for r in rows.values()) * bench.NCLASS * 4 <= bench.DUMP_PROB_BYTES <= 48 << 20
+    for world in (1, 2, 8):
+        st = [bench.dump_rows(e - b, world, rank) for rank, (b, e) in enumerate(row_partition(bench.ST_ROWS, world))]
+        assert sum(r.size for r in st) * bench.NCLASS * 4 <= bench.DUMP_PROB_BYTES
+    assert bench.dump_rows(bench.ST_ROWS // 2, 2, 1)[:4].tolist() == [5, 7, 9, 22]
+    assert np.array_equal(bench.dump_rows(10, 23, 0), np.arange(10))          # small graphs are written whole
+
+
 def test_reference_arm_runs_on_the_host_and_prints_one_line():
     env = dict(os.environ, OMP_NUM_THREADS="4")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "c1", "--steps", "1",
