@@ -26,8 +26,6 @@
 // ~156 KB of L1.  That matters more than anything else in this kernel: every in-flight gather load holds an L1 line,
 // and the first version (weight image resident in shared memory, 225 KB, ~28 KB of L1) ran the gather at 0.4 of the
 // standalone SpMM's rate for exactly that reason (profiles/r02_fused_v1_*).
-#include <cstdlib>
-
 #include "common.cuh"
 #include "tc_ptx.cuh"
 #include "fused_layer.cuh"
@@ -38,12 +36,9 @@ namespace fl {
 using namespace tc;
 
 constexpr int TM = 64;                         // panel rows per tile = UMMA N
-// Epilogue warps E (4 or 8; warps 0..3 are the ones that read the accumulator, warp w <-> TMEM lane quarter w) come
-// first, then the gather / producer warps; the first of those also issues the MMAs (no dedicated warp).  Registers per
-// thread follow from the warps per scheduler: 20 warps -> 96, 24 warps -> 80.
-constexpr int threads_for(int gw, int e) { return (e + gw) * 32; }
-// Gather warps per CTA: 16 (640 threads, 96 registers, 2 x 4 column indices x strands of loads in flight per warp) or
-// 8 (384 threads, 168 registers, 2 x 8).  CGCN_FUSED_GW selects; both are built.
+// The E = 4 epilogue warps (warp w <-> TMEM lane quarter w) come first, then the 16 gather warps; the first of those also
+// issues the MMAs (no dedicated warp).  20 warps = 5 per scheduler -> 96 registers per thread.
+constexpr int E = 4, G_WARPS = 16, THREADS = (E + G_WARPS) * 32;
 constexpr int A_CHUNK = TM * 128;              // one k-chunk (32 floats) of the tile: 64 rows x 128 B = 8 KB
 constexpr int A_BYTES = 2 * 4 * A_CHUNK;       // hi + lo: 64 KB
 constexpr int Y_BYTES = TM * 512;              // fp32 y tile, row major [64 rows][128 features]: 32 KB
@@ -108,8 +103,8 @@ __device__ __forceinline__ float4 lds_f4(uint32_t saddr) {
   return make_float4(__uint_as_float(v.x), __uint_as_float(v.y), __uint_as_float(v.z), __uint_as_float(v.w));
 }
 
-template <int S, int MODE, int G_WARPS, bool PEER, int SRC, int E>
-__global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel(const Args a) {
+template <int S, int MODE, bool PEER>
+__global__ void __launch_bounds__(THREADS, 1) fused_layer_kernel(const Args a) {
   constexpr int EPI_WARPS = E, ISSUE_WARP = E;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t base = smem_u32(smem_raw);
@@ -171,15 +166,12 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
     }
     tmem_wait_st();
     tc_fence_before();
-    if constexpr (E != 8) {                        // E == 8: after these warps have given registers back (see below)
-      named_bar_sync(3, 5 * 32);
-      tc_fence_after();
-    }
+    named_bar_sync(3, 5 * 32);
+    tc_fence_after();
   }
 
   if (warp >= EPI_WARPS) {
     // =========================================================== gather warps
-    if constexpr (E == 8) asm volatile("setmaxnreg.inc.sync.aligned.u32 88;");
     // Each warp owns RPW window rows of every tile and walks their neighbour lists as ONE stream of "segments" (<= 32
     // column indices of one row, held one per lane) cut into batches of U neighbours.  Two register sets alternate:
     // while batch i is being summed, batch i+1 -- of the same segment, or the first of the next row / tile -- is already
@@ -216,8 +208,6 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
       }
       __syncwarp();
     };
-
-
     // one finished panel row (lane owns columns 4 lane .. 4 lane + 3) into the tile buffer as hi / lo TF32
     auto put_row = [&](int pr, const float4 v) {
       uint4 hi, lo;
@@ -233,74 +223,7 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
       if (warp == ISSUE_WARP) issue_mma(t);
     };
 
-    if constexpr (SRC != GATHER) {
-      // ---- streaming producer: the tile is rows of gsrc (already aggregated by the SpMM, or the head's input), NT tiles
-      // of look-ahead in a register ring: 12 coalesced 512-byte loads in flight per warp, continuously
-      constexpr int NT = 3, RP = RPW * S;
-      float4 ring[NT][RP];
-      int ring_deg[NT][RPW];
-      auto load_tile = [&](int t, float4 (&b)[RP], int (&dg)[RPW]) {
-#pragma unroll
-        for (int h = 0; h < RPW; ++h) {
-          const int row = r_begin + t * TG + gw + G_WARPS * h;
-          const bool valid = t < ntile && row < r_end;
-          dg[h] = 1;
-          if (FORWARD && SRC == STREAM && valid) dg[h] = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row);
-#pragma unroll
-          for (int s = 0; s < S; ++s)
-            b[h * S + s] = valid ? ldg4(a.gsrc + (static_cast<size_t>(row) * S + s) * 128 + lane * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      };
-      float4 bn_m[S], bn_r[S], bn_g = make_float4(0.f, 0.f, 0.f, 0.f), bn_b = bn_g;
-      if constexpr (SRC == STREAM_BN) {
-        bn_g = ldg4(a.bn_gamma + lane * 4);
-        bn_b = ldg4(a.bn_beta + lane * 4);
-#pragma unroll
-        for (int s = 0; s < S; ++s) {
-          bn_m[s] = ldg4(a.bn_mean + s * 128 + lane * 4);
-          bn_r[s] = ldg4(a.bn_rstd + s * 128 + lane * 4);
-        }
-      }
-#pragma unroll
-      for (int j = 0; j < NT; ++j) load_tile(j, ring[j], ring_deg[j]);
-#pragma unroll 1
-      for (int t0 = 0; t0 < ntile; t0 += NT) {
-#pragma unroll
-        for (int j = 0; j < NT; ++j) {
-          const int t = t0 + j;
-          if (t < ntile) {
-            mbar_wait(bar_a_empty, (t & 1) ^ 1);
-#pragma unroll
-            for (int h = 0; h < RPW; ++h) {
-              const int lr = gw + G_WARPS * h;
-              const int row = r_begin + t * TG + lr;
-              float scale = 1.0f;
-              if (FORWARD && SRC == STREAM) scale = ring_deg[j][h] > 0 ? __fdiv_rn(1.0f, static_cast<float>(ring_deg[j][h])) : 1.0f;
-#pragma unroll
-              for (int s = 0; s < S; ++s) {
-                float4 v = ring[j][h * S + s];
-                if constexpr (SRC == STREAM_BN) {
-                  v = make_float4((fmaxf(v.x, 0.f) - bn_m[s].x) * bn_r[s].x * bn_g.x + bn_b.x, (fmaxf(v.y, 0.f) - bn_m[s].y) * bn_r[s].y * bn_g.y + bn_b.y,
-                                  (fmaxf(v.z, 0.f) - bn_m[s].z) * bn_r[s].z * bn_g.z + bn_b.z, (fmaxf(v.w, 0.f) - bn_m[s].w) * bn_r[s].w * bn_g.w + bn_b.w);
-                  const size_t ofs = (static_cast<size_t>(row) * S + s) * 128 + lane * 4;
-                  if (a.drop.enabled) {
-                    const float4 m = dropout_mult4(a.drop, ofs >> 2);
-                    v = make_float4(v.x * m.x, v.y * m.y, v.z * m.z, v.w * m.w);
-                  }
-                  if (row < r_end) st4(a.hb_out + ofs, v);
-                } else {
-                  v = make_float4(v.x * scale, v.y * scale, v.z * scale, v.w * scale);
-                }
-                put_row(lr * S + s, v);
-              }
-            }
-            deliver(t);
-            load_tile(t + NT, ring[j], ring_deg[j]);
-          }
-        }
-      }
-    } else {
-    constexpr int U = (G_WARPS == 8) ? ((S == 2) ? 8 : 12) : ((S == 2) ? 3 : 6);
+    constexpr int U = (S == 2) ? 3 : 6;
     const int nrow = ntile * RPW;                  // rows this warp visits; rows beyond r_end read as empty
     auto load_ptrs = [&](int t) -> int {           // lane 2h + e holds rowptr[row_h + e] of tile t
       int v = 0;
@@ -404,22 +327,11 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
         if (h == 0) mbar_wait(bar_a_empty, (t & 1) ^ 1);        // the MMAs of the previous tile have read the tile buffer
 #pragma unroll
         for (int s = 0; s < S; ++s) {
-          const int pr = lr * S + s;
-          const float4 v = make_float4(acc[s].x * scale, acc[s].y * scale, acc[s].z * scale, acc[s].w * scale);
-          uint4 hi, lo;
-          split4(v, hi, lo);
-          const uint32_t off = (lane >> 3) * A_CHUNK + (pr >> 3) * 1024 + (pr & 7) * 128 + (((lane & 7) ^ (pr & 7)) << 4);
-          sts128(sA + off, hi);
-          sts128(sA + 4 * A_CHUNK + off, lo);
+          put_row(lr * S + s, make_float4(acc[s].x * scale, acc[s].y * scale, acc[s].z * scale, acc[s].w * scale));
           acc[s] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
         deg = 0;
-        if (h == RPW - 1) {
-          fence_async_smem();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(bar_a_full);
-          if (warp == ISSUE_WARP) issue_mma(t);
-        }
+        if (h == RPW - 1) deliver(t);
         ++q;
       }
       c_cols = n_cols;
@@ -428,27 +340,13 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
       n_cl = nn_cl;
       next_seg(nn_cols, nn_cl);
     }
-    }
   } else {
     // =========================================================== epilogue warps
-    if constexpr (E == 8) {
-      // 24 warps start at 80 registers; the epilogue warps drop to 64 so that the 16 gather warps can grow to 88.
-      // setmaxnreg.inc draws only on what warps of this CTA have released (SASS: USETMAXREG.TRY_ALLOC.CTAPOOL), not on
-      // registers the launch left unallocated: 8 x 16 released = 16 x 8 acquired; asking for more (56 / 96, 64 / 96)
-      // spins forever.  The weight-image warps release theirs BEFORE they wait for the issuing warp on barrier 3: that
-      // warp may itself be waiting for these registers.
-      asm volatile("setmaxnreg.dec.sync.aligned.u32 64;");
-      if (warp < 4 && ntile > 0) {
-        named_bar_sync(3, 5 * 32);
-        tc_fence_after();
-      }
-    }
     // Phase A (thread = output feature: the accumulator is y^T, TMEM lane f = feature f, column r = tile row r):
     // TMEM -> + bias -> row-major shared y tile (one conflict-free 128-byte store per row per warp).
     // Phase B (LPR lanes per row, RPI rows per warp step; lane q owns the float4 column groups cc * CSTRIDE + 4 q):
-    // everything else, on TM / E rows per epilogue warp.  E = 4: 8 lanes per row, 16 values per lane per step;
-    // E = 8: 16 lanes per row, 8 values per lane (fits the 80-register budget of a 24-warp CTA).
-    constexpr int LPR = (E == 4) ? 8 : 16, RPI = 32 / LPR, CPL = 32 / LPR, CSTRIDE = LPR * 4;
+    // everything else, on TM / E rows per epilogue warp: 8 lanes per row, 16 values per lane per step.
+    constexpr int LPR = 8, RPI = 32 / LPR, CPL = 32 / LPR, CSTRIDE = LPR * 4;
     constexpr int ROWS_W = TM / E, ITERS = ROWS_W / RPI;
     static_assert(CPL * CSTRIDE == 128 && ITERS >= 1 && ROWS_W % 2 == 0 && E * RPI == 16, "epilogue split");
     const int sub = lane / LPR, q = lane % LPR;
@@ -460,7 +358,6 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
     const float bg = (FORWARD && !a.gate_off) ? __ldg(a.bg) : 0.f;
     float bias_f = 0.f;                            // threadIdx.x = this thread's feature
     if (FORWARD && threadIdx.x < 128) bias_f = __ldg(a.bias + threadIdx.x);
-    if (MODE == HEAD_FWD && static_cast<int>(threadIdx.x) < a.w_rows) bias_f = __ldg(a.bias + threadIdx.x);
     const int64_t prow_end = static_cast<int64_t>(r_end) * S;
 
     for (int t = 0; t < ntile; ++t) {
@@ -501,7 +398,7 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
             for (int cc = 0; cc < CPL; ++cc) {
               if constexpr (FORWARD) {
                 prefetch_l1(a.xin + nofs + cc * CSTRIDE);
-              } else if constexpr (MODE != HEAD_FWD) {
+              } else {
                 prefetch_l1(a.dxd_in + nofs + cc * CSTRIDE);
                 if constexpr (MODE == BWD_MID) {
                   prefetch_l1(a.z_prev + nofs + cc * CSTRIDE);
@@ -529,7 +426,6 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
           dot += __shfl_xor_sync(0xffffffffu, dot, 1);
           dot += __shfl_xor_sync(0xffffffffu, dot, 2);
           dot += __shfl_xor_sync(0xffffffffu, dot, 4);
-          if (LPR == 16) dot += __shfl_xor_sync(0xffffffffu, dot, 8);
           const float g = a.gate_off ? 1.0f : sigmoidf_(dot + bg);
           const float omg = 1.0f - g;
           if (valid) {
@@ -550,12 +446,6 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
                 st1[cc].x += rl.x * rl.x; st1[cc].y += rl.y * rl.y; st1[cc].z += rl.z * rl.z; st1[cc].w += rl.w * rl.w;
               }
             }
-          }
-        } else if constexpr (MODE == HEAD_FWD) {     // logits: the first out_ld columns of the row (bias added in phase A)
-          if (valid) {
-#pragma unroll
-            for (int cc = 0; cc < CPL; ++cc)
-              if (cc * CSTRIDE + 4 * q < a.out_ld) st4(a.out + static_cast<size_t>(grow) * a.out_ld + cc * CSTRIDE + 4 * q, y[cc]);
           }
         } else if constexpr (MODE == BWD_INPUT) {
           if (valid) {
@@ -596,7 +486,6 @@ __global__ void __launch_bounds__(threads_for(G_WARPS, E), 1) fused_layer_kernel
           part += __shfl_xor_sync(0xffffffffu, part, 1);
           part += __shfl_xor_sync(0xffffffffu, part, 2);
           part += __shfl_xor_sync(0xffffffffu, part, 4);
-          if (LPR == 16) part += __shfl_xor_sync(0xffffffffu, part, 8);
           if (valid) {
             const float dgp = a.gate_off ? 0.0f : part * g * (1.0f - g);
             const float omg = 1.0f - g;
@@ -695,45 +584,39 @@ int fused_layer_grid(int n, int S, int* rows_per_cta_out) {
 
 bool fused_layer_supported(int d, const cgcn_graph* g) { return d == 128 && g != nullptr && g->vals == nullptr; }
 
+template <int S, int MODE, bool PEER>
+static int launch_kernel(const fl::Args& a, int grid, cudaStream_t stream) {
+  static bool attr_set[64] = {};
+  if (first_use_on_device(attr_set))
+    CGCN_CUDA(cudaFuncSetAttribute(fl::fused_layer_kernel<S, MODE, PEER>, cudaFuncAttributeMaxDynamicSharedMemorySize, fl::SMEM));
+  CGCN_CUDA(launch_k(fl::fused_layer_kernel<S, MODE, PEER>, dim3(grid), dim3(fl::THREADS), fl::SMEM, stream, a));
+  return check_launch("fused_layer_kernel");
+}
+
+template <int S, bool PEER>
+static int launch_mode(const fl::Args& a, int mode, int grid, cudaStream_t stream) {
+  switch (mode) {
+    case fl::FWD: return launch_kernel<S, fl::FWD, PEER>(a, grid, stream);
+    case fl::FWD_STATS: return launch_kernel<S, fl::FWD_STATS, PEER>(a, grid, stream);
+    case fl::BWD_MID: return launch_kernel<S, fl::BWD_MID, PEER>(a, grid, stream);
+    case fl::BWD_INPUT: return launch_kernel<S, fl::BWD_INPUT, PEER>(a, grid, stream);
+  }
+  set_error("fused layer: unsupported strands=%d mode=%d", S, mode);
+  return CGCN_ERR_INVALID;
+}
+
 int fused_layer_launch(fl::Args a, int S, int mode, int* grid_out, cudaStream_t stream) {
-  CGCN_REQUIRE((a.source != fl::GATHER || (a.rowptr && a.colidx)) && (a.gsrc || a.peer_world > 0) && a.w,
-               "fused layer: null graph / panel / weight");
+  CGCN_REQUIRE(a.rowptr && a.colidx && (a.gsrc || a.peer_world > 0) && a.w, "fused layer: null graph / panel / weight");
   CGCN_REQUIRE(S == 1 || S == 2, "fused layer: strands=%d", S);
   int rows = 0;
   const int grid = fused_layer_grid(a.n, S, &rows);
   a.rows_per_cta = rows;
   if (grid_out) *grid_out = grid;
   if (a.n <= 0) return CGCN_OK;
-  static const int gw = (getenv("CGCN_FUSED_GW") != nullptr && atoi(getenv("CGCN_FUSED_GW")) == 8) ? 8 : 16;
   const bool peer = a.peer_world > 0;
   if (peer) a.gsrc = a.peer_base[0];
-  const int src = a.source;
-  CGCN_REQUIRE(!(peer && src != fl::GATHER), "fused layer: peer panels are gathered, not streamed");
-  CGCN_REQUIRE((mode == fl::HEAD_FWD) == (src == fl::STREAM_BN), "fused layer: HEAD_FWD goes with STREAM_BN");
-#define FL_LAUNCH(SV, MV, GV, PV, RV, EV)                                                                            \
-  if (S == SV && mode == MV && gwsel == GV && peer == PV && src == RV && esel == EV) {                               \
-    static bool attr_set[64] = {};                                                                                   \
-    if (first_use_on_device(attr_set))                                                                               \
-      CGCN_CUDA(cudaFuncSetAttribute(fl::fused_layer_kernel<SV, MV, GV, PV, RV, EV>, cudaFuncAttributeMaxDynamicSharedMemorySize, fl::SMEM)); \
-    CGCN_CUDA(launch_k(fl::fused_layer_kernel<SV, MV, GV, PV, RV, EV>, dim3(grid), dim3(fl::threads_for(GV, EV)), fl::SMEM, stream, a)); \
-    return check_launch("fused_layer_kernel");                                                                      \
-  }
-  const int gwsel = (src == fl::GATHER) ? gw : 16;
-  static const int e_env = getenv("CGCN_FUSED_EPI") != nullptr ? atoi(getenv("CGCN_FUSED_EPI")) : 4;
-  const int esel = (gwsel == 16 && !peer && e_env == 8) ? 8 : 4;
-#define FL_MODES(SV, GV, PV, RV, EV) \
-  FL_LAUNCH(SV, fl::FWD, GV, PV, RV, EV) FL_LAUNCH(SV, fl::FWD_STATS, GV, PV, RV, EV) FL_LAUNCH(SV, fl::BWD_MID, GV, PV, RV, EV) FL_LAUNCH(SV, fl::BWD_INPUT, GV, PV, RV, EV)
-#define FL_STRANDS(SV)                                                                                              \
-  FL_MODES(SV, 16, false, fl::GATHER, 4) FL_MODES(SV, 16, false, fl::GATHER, 8) FL_MODES(SV, 16, true, fl::GATHER, 4) \
-  FL_MODES(SV, 8, false, fl::GATHER, 4) FL_MODES(SV, 16, false, fl::STREAM, 4) FL_MODES(SV, 16, false, fl::STREAM, 8) \
-  FL_LAUNCH(SV, fl::HEAD_FWD, 16, false, fl::STREAM_BN, 4) FL_LAUNCH(SV, fl::HEAD_FWD, 16, false, fl::STREAM_BN, 8)
-  FL_STRANDS(1)
-  FL_STRANDS(2)
-#undef FL_LAUNCH
-#undef FL_MODES
-#undef FL_STRANDS
-  set_error("fused layer: unsupported strands=%d mode=%d", S, mode);
-  return CGCN_ERR_INVALID;
+  if (S == 1) return peer ? launch_mode<1, true>(a, mode, grid, stream) : launch_mode<1, false>(a, mode, grid, stream);
+  return peer ? launch_mode<2, true>(a, mode, grid, stream) : launch_mode<2, false>(a, mode, grid, stream);
 }
 
 int fused_layer_set_peer(fl::Args* a, const cgcn_peer_panel* pp, int n_local) {

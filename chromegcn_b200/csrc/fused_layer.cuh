@@ -5,11 +5,7 @@
 namespace cgcn {
 namespace fl {
 
-enum Mode { FWD = 0, FWD_STATS = 1, BWD_MID = 2, BWD_INPUT = 3, HEAD_FWD = 4 };
-// Where the 64-row operand tile comes from: GATHER = CSR gather-reduce of gsrc inside the kernel; STREAM = the rows of
-// gsrc as they are (the aggregation was done by the standalone SpMM; forward: scaled by 1/deg here); STREAM_BN = the rows
-// of gsrc through relu -> BatchNorm -> dropout (the head of models/ChromeModels.py:48-50), also written to hb_out.
-enum Source { GATHER = 0, STREAM = 1, STREAM_BN = 2 };
+enum Mode { FWD = 0, FWD_STATS = 1, BWD_MID = 2, BWD_INPUT = 3 };
 
 struct Args {
   const int32_t* rowptr;
@@ -39,16 +35,6 @@ struct Args {
   float* dys_out;              // D^-1 dy_{l-1}
   float* dxd_out;              // (1-g_{l-1}) dh_{l-1} or NULL (may alias dxd_in)
   float* dx_out;               // BWD_INPUT: d loss / d x_in
-  // ---- head (HEAD_FWD + STREAM_BN): out = dropout(BatchNorm(relu(gsrc))) Wout^T + bout
-  int source;                  // fl::Source
-  int w_rows;                  // valid rows of a transposed weight operand (nclass for the head; 0 = 128)
-  const float* bn_mean;        // [S][128]
-  const float* bn_rstd;        // [S][128]
-  const float* bn_gamma;       // [128]
-  const float* bn_beta;        // [128]
-  float* hb_out;               // [n][S][128] the transformed rows (saved for d Wout = dout^T hb)
-  float* out;                  // [n][S][out_ld] logits
-  int out_ld;
   // ---- peer gather (one graph row-partitioned over the GPUs of an NVLink box): the gathered panel lives in the ranks'
   // exchange buffers (cgcn_peer_panel); rank r owns global rows [peer_begin[r], peer_begin[r+1]) at peer_base[r].
   // peer_world == 0: plain gather from gsrc.

@@ -354,9 +354,8 @@ struct GramTcArgs {
 constexpr int GR_OP_BYTES = 2 * CHUNK_BYTES;                     // one operand, hi + lo, 32 rows x 128 cols: 32 KB
 constexpr int GR_STAGE_BYTES = 2 * GR_OP_BYTES;                  // A + B: 64 KB
 constexpr int GR_SMEM = STAGES * GR_STAGE_BYTES + STG_BYTES + 256 + 1024;
+constexpr int GR_SLOTS = 2;                                      // register look-ahead of the producers, in 32-row chunks
 
-// GR_SLOTS: register look-ahead of the producers, in 32-row chunks
-template <int GR_SLOTS>
 __global__ void __launch_bounds__(THREADS, 1) gemm_gram_tc_kernel(const GramTcArgs p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -592,11 +591,9 @@ int gemm_gram_tc(const float* A, int64_t lda, const float* B, int64_t ldb, float
     set_error("cgcn_gemm_gram(tcgen05): workspace %zu < %zu bytes", workspace_bytes, gram_workspace_bytes(m));
     return CGCN_ERR_WORKSPACE;
   }
-  static const int slots = getenv("CGCN_GRAM_SLOTS") ? atoi(getenv("CGCN_GRAM_SLOTS")) : 2;   // developer aid: 3 chunks of look-ahead measured no faster (15.85 vs 15.79 ms per pass)
   static bool attr_set[64] = {};
   if (first_use_on_device(attr_set)) {
-    CGCN_CUDA(cudaFuncSetAttribute(tc::gemm_gram_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::GR_SMEM));
-    CGCN_CUDA(cudaFuncSetAttribute(tc::gemm_gram_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::GR_SMEM));
+    CGCN_CUDA(cudaFuncSetAttribute(tc::gemm_gram_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::GR_SMEM));
   }
   // one CTA per SM (the kernel owns the whole shared memory): a single wave, <= #SM partial tiles
   int64_t rows = (m + sm_count() - 1) / sm_count();
@@ -604,10 +601,7 @@ int gemm_gram_tc(const float* A, int64_t lda, const float* B, int64_t ldb, float
   rows = (rows + tc::KCH - 1) / tc::KCH * tc::KCH;
   const int parts = static_cast<int>((m + rows - 1) / rows);
   tc::GramTcArgs p{A, lda, B, ldb, m, rows, static_cast<float*>(workspace), ka, nb};
-  if (slots == 2)
-    CGCN_CUDA(launch_k(tc::gemm_gram_tc_kernel<2>, dim3(parts), dim3(tc::THREADS), tc::GR_SMEM, stream, p));
-  else
-    CGCN_CUDA(launch_k(tc::gemm_gram_tc_kernel<3>, dim3(parts), dim3(tc::THREADS), tc::GR_SMEM, stream, p));
+  CGCN_CUDA(launch_k(tc::gemm_gram_tc_kernel, dim3(parts), dim3(tc::THREADS), tc::GR_SMEM, stream, p));
   CGCN_TRY(check_launch("gemm_gram_tc_kernel"));
   gram_finalize_launch(p.partial, parts, tc::TILE * tc::TILE, tc::TILE, ka, nb, C, ldc, accumulate, stream);
   return check_launch("gram_finalize_kernel");

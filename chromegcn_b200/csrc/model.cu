@@ -352,34 +352,17 @@ static const void* bwd_image(const Ctx& c, int i) { return use_images(c.m) ? c.w
 
 // The fused layer kernels (fused_layer.cu): one launch per layer and direction instead of SpMM + contraction + gate
 // kernel.  In this mode the saved `ax` panels hold the UN-normalised neighbour sums and the `dy` panels hold
-// D^-1 dy, so that d W = ax^T dy is unchanged while the backward gather needs no per-neighbour scale.
-// Layer modes: 0 = three kernels per layer (SpMM, row-panel contraction, gate kernel); 1 = "gather" (default for Hi-C
-// degrees): everything in one kernel, CSR gather included; 2 = "stream": the standalone SpMM + ONE kernel for contraction,
-// gate, blend, dropout and column partials, its operand tile streamed from the SpMM's output.  Modes 1 and 2 share the
-// conventions above.  Measured on B200, whole genome (mean degree 10.7), ms per pass: unfused 16.9, gather 16.0 -> 15.7,
-// stream 18.2 (profiles/r02_layer_modes.md): the contraction + epilogue kernel is bound by its four epilogue warps
-// (one per scheduler), not by where its operand comes from.  The all-in-one kernel keeps ~200 gather loads in flight per
+// D^-1 dy, so that d W = ax^T dy is unchanged while the backward gather needs no per-neighbour scale.  A fused forward
+// is always followed by the fused backward.  Measured on B200, whole genome (mean degree 10.7), ms per pass: three
+// kernels 16.9, fused 15.7 (profiles/r02_layer_modes.md).  The all-in-one kernel keeps ~200 gather loads in flight per
 // SM against the SpMM's ~320, so once the gather dominates (mean degree 51: fused 6.5 ms per layer vs SpMM 2.15 + 0.6 +
-// 0.9) mode 0 wins: graphs beyond CGCN_FUSED_MAX_DEGREE (default 24) stored entries per row use it.
-static int layer_mode(const cgcn_model* m) {
-  static const char* env = getenv("CGCN_LAYER_MODE");              // "unfused" | "gather" | "stream"
+// 0.9) the three kernels win: graphs with more than FUSED_MAX_DEGREE stored entries per row on average use them.
+constexpr int64_t FUSED_MAX_DEGREE = 24;
+static bool use_fused(const cgcn_model* m) {
   static const bool off = getenv("CGCN_NO_FUSED") != nullptr;       // developer aid / A-B measurements
-  if (off || !use_images(m) || !fused_layer_supported(m->d, &m->graph)) return 0;
-  if (env != nullptr && strcmp(env, "unfused") == 0) return 0;
-  if (env != nullptr && strcmp(env, "stream") == 0) return 2;
-  if (env != nullptr && strcmp(env, "gather") == 0) return 1;
-  static const int max_deg = getenv("CGCN_FUSED_MAX_DEGREE") ? atoi(getenv("CGCN_FUSED_MAX_DEGREE")) : 24;
+  if (off || !use_images(m) || !fused_layer_supported(m->d, &m->graph)) return false;
   const int64_t nnz = m->graph.nnz, n = m->graph.n > 0 ? m->graph.n : 1;
-  return nnz <= static_cast<int64_t>(max_deg) * n ? 1 : 0;
-}
-static bool use_fused(const cgcn_model* m) { return layer_mode(m) != 0; }
-// The backward twin of the fused kernel (gather -> W^T -> + (1-g) dh -> gate backward of the layer below) measures the
-// same as row-panel contraction + SpMM + gate kernel on the fused forward's conventions (15.7 ms per whole-genome pass
-// either way: it is bound by its four epilogue warps streaming three panels); it is the default because it moves 5
-// panels instead of 9.  CGCN_BWD_UNFUSED=1 selects the three kernels.
-static bool use_fused_bwd(const cgcn_model* m) {
-  static const bool off = getenv("CGCN_BWD_UNFUSED") != nullptr;
-  return !off && use_fused(m);
+  return nnz <= FUSED_MAX_DEGREE * n;
 }
 
 static int prep_fwd_images(const Ctx& c) {
@@ -432,18 +415,8 @@ static int fwd_layer(const Ctx& c, int l, const float* gather_src) {
     a.rowptr = m->graph.rowptr;
     a.colidx = m->graph.colidx;
     a.n = c.n;
-    if (layer_mode(m) == 2) {
-      // sx = P x by the SpMM kernel (un-normalised sums), then the contraction + epilogue kernel streams it
-      if (c.dist && m->peer != nullptr)
-        CGCN_TRY(spmm_peer_launch(&m->graph, m->peer, ws + lay.ax[l], c.W, 0, nullptr, c.st));
-      else
-        CGCN_TRY(spmm_launch(&m->graph, gather_src, ws + lay.ax[l], c.W, 0, nullptr, c.st));
-      a.source = fl::STREAM;
-      a.gsrc = ws + lay.ax[l];
-    } else {
-      a.gsrc = gather_src;
-      if (c.dist && m->peer != nullptr) CGCN_TRY(fused_layer_set_peer(&a, m->peer, c.n));      // neighbour rows over NVLink
-    }
+    a.gsrc = gather_src;
+    if (c.dist && m->peer != nullptr) CGCN_TRY(fused_layer_set_peer(&a, m->peer, c.n));      // neighbour rows over NVLink
     a.w = m->params.gc_w[l];
     a.w_transposed = 0;
     a.xin = xin;
@@ -494,28 +467,6 @@ static int fwd_head(const Ctx& c) {
     CGCN_TRY(bn_finalize_launch(ws + lay.partial, 0, c.n_total, c.S, c.d, m->bn_eps, m->bn_momentum, m->training,
                                 m->bn_running_mean, m->bn_running_var, m->bn_num_batches_tracked, ws + lay.bn_mean,
                                 ws + lay.bn_rstd, m->training ? m->bn_sums : nullptr, nullptr, c.st));
-  const int ldo_f = m->out_ld > 0 ? m->out_ld : c.C;
-  static const bool fused_head = getenv("CGCN_FUSED_HEAD") != nullptr;      // measured 62.6 us vs 27 + 29 for the two kernels below
-  if (fused_head && use_fused(m) && ldo_f % 4 == 0) {
-    // hb = dropout(BatchNorm(relu(x))) in the producer warps, out = hb Wout^T + bout on the tensor cores: one kernel
-    fl::Args a{};
-    a.n = c.n;
-    a.source = fl::STREAM_BN;
-    a.gsrc = ws + lay.xo[c.L - 1];
-    a.bn_mean = ws + lay.bn_mean;
-    a.bn_rstd = ws + lay.bn_rstd;
-    a.bn_gamma = m->params.bn_w;
-    a.bn_beta = m->params.bn_b;
-    a.hb_out = ws + lay.hb;
-    a.drop = make_dropout(m->dropout_p, m->seed, m->step, 1, m->training, c.drop_off);
-    a.w = m->params.out_w;
-    a.w_transposed = 1;
-    a.w_rows = c.C;
-    a.bias = m->params.out_b;
-    a.out = m->out;
-    a.out_ld = ldo_f;
-    return fused_layer_launch(a, c.S, fl::HEAD_FWD, nullptr, c.st);
-  }
   // hb = dropout(BatchNorm(relu(x)))                 (models/ChromeModels.py:48-50)
   BnApplyArgs b{};
   b.h = ws + lay.xo[c.L - 1];
@@ -637,19 +588,8 @@ static int bwd_propagate_fused(const Ctx& c, int l_from, const float* gather_src
   a.rowptr = m->graph.rowptr;
   a.colidx = m->graph.colidx;
   a.n = c.n;
-  if (layer_mode(m) == 2) {
-    // u = P dys by the SpMM kernel into a scratch panel (dX: the head's d hb, dead since its gate stage)
-    float* u = ws + lay.dX;
-    if (c.dist && m->peer != nullptr)
-      CGCN_TRY(spmm_peer_launch(&m->graph, m->peer, u, c.W, 0, nullptr, c.st));
-    else
-      CGCN_TRY(spmm_launch(&m->graph, gather_src, u, c.W, 0, nullptr, c.st));
-    a.source = fl::STREAM;
-    a.gsrc = u;
-  } else {
-    a.gsrc = gather_src;
-    if (c.dist && m->peer != nullptr) CGCN_TRY(fused_layer_set_peer(&a, m->peer, c.n));
-  }
+  a.gsrc = gather_src;
+  if (c.dist && m->peer != nullptr) CGCN_TRY(fused_layer_set_peer(&a, m->peer, c.n));
   a.w = m->params.gc_w[l_from];
   a.w_transposed = 1;
   a.dxd_in = ws + lay.dC;
@@ -717,7 +657,7 @@ static int bwd_layer_fused(const Ctx& c, Fork& f, int l, int parts, const float*
 
 // gate stage of layer l, its weight gradients (side stream) and, if anything upstream needs it, t = D^-1 (dy W^T).
 // Returns in *t_out the panel holding t (NULL if the chain stops here).
-static int bwd_layer(const Ctx& c, Fork& f, int l, const float** t_out, bool dys = false) {
+static int bwd_layer(const Ctx& c, Fork& f, int l, const float** t_out) {
   const cgcn_model* m = c.m;
   const WsLayout& lay = c.lay;
   float* ws = c.ws;
@@ -746,9 +686,6 @@ static int bwd_layer(const Ctx& c, Fork& f, int l, const float** t_out, bool dys
   a.partial = ws + lay.partial_l[l];
   a.n = c.n;
   a.drop = make_dropout(m->dropout_p, m->seed, m->step, head ? 1 : layer_drop_site(l), m->training, c.drop_off);
-  // dys: the forward pass was fused (saved panels hold the UN-normalised sums), so dy is stored as D^-1 dy: the weight
-  // gradient ax^T dy keeps its value and the contraction below needs no row scale ((D^-1 dy) W^T = D^-1 (dy W^T))
-  a.scale_rowptr = dys ? m->graph.rowptr : nullptr;
   int grid = 0;
   CGCN_TRY(gate_bwd_launch(a, c.d, c.S, head, &grid, c.st));
   // side: bias / gate gradients from the partials, d W = (A_hat x)^T dy
@@ -758,8 +695,8 @@ static int bwd_layer(const Ctx& c, Fork& f, int l, const float** t_out, bool dys
                               lay.gram_bytes, f.ss));
   if (!need_dx) return CGCN_OK;
   // main: t = D^-1 (dy W^T) -> the panel that held `src`
-  CGCN_TRY(gemm_rowpanel_dispatch(dy, c.d, m->params.gc_w[l], 1, nullptr, src, c.d, c.M, c.d, c.d, dys ? nullptr : m->graph.rowptr,
-                                  dys ? nullptr : m->graph.row_inv, c.S, m->gemm_impl, c.tcws, lay.tc_bytes, c.st, bwd_image(c, 1 + l)));
+  CGCN_TRY(gemm_rowpanel_dispatch(dy, c.d, m->params.gc_w[l], 1, nullptr, src, c.d, c.M, c.d, c.d, m->graph.rowptr,
+                                  m->graph.row_inv, c.S, m->gemm_impl, c.tcws, lay.tc_bytes, c.st, bwd_image(c, 1 + l)));
   *t_out = src;
   return CGCN_OK;
 }
@@ -771,8 +708,7 @@ static int model_backward(const cgcn_model* m) {
   Fork f;
   CGCN_TRY(make_fork(c, &f));
   CGCN_TRY(bwd_head(c, f));
-  const bool dys = use_fused(m);
-  if (use_fused_bwd(m)) {
+  if (use_fused(m)) {
     int parts = 0;
     for (int l = c.L - 1; l >= 0; --l) {
       const float* t = nullptr;
@@ -784,7 +720,7 @@ static int model_backward(const cgcn_model* m) {
   }
   for (int l = c.L - 1; l >= 0; --l) {
     const float* t = nullptr;
-    CGCN_TRY(bwd_layer(c, f, l, &t, dys));
+    CGCN_TRY(bwd_layer(c, f, l, &t));
     if (t == nullptr) break;
     CGCN_TRY(bwd_propagate(c, l, t));
   }
@@ -819,19 +755,19 @@ static int model_phase(const cgcn_model* m, int kind, int layer, const float** p
     case CGCN_PHASE_BWD_HEAD:
       return bwd_head(c, f);
     case CGCN_PHASE_BWD_LAYER:       // layer == L-1: bn_sums all-reduced ; else: x_full holds the gathered t of layer+1
-      if (use_fused_bwd(m)) {
+      if (use_fused(m)) {
         int parts = 0;
         if (layer < c.L - 1) CGCN_TRY(bwd_propagate_fused(c, layer + 1, m->x_full, &parts));
         CGCN_TRY(bwd_layer_fused(c, f, layer, parts, &t));
       } else {
         if (layer < c.L - 1) CGCN_TRY(bwd_propagate(c, layer + 1, m->x_full));
-        CGCN_TRY(bwd_layer(c, f, layer, &t, use_fused(m)));
+        CGCN_TRY(bwd_layer(c, f, layer, &t));
       }
       if (publish) *publish = t;
       return CGCN_OK;
     case CGCN_PHASE_BWD_INPUT:       // x_full holds the gathered t of layer 0
       CGCN_REQUIRE(m->need_input_grad && m->x_in_grad, "cgcn_model_phase: BWD_INPUT without need_input_grad");
-      if (use_fused_bwd(m)) return bwd_propagate_fused(c, 0, m->x_full, nullptr);
+      if (use_fused(m)) return bwd_propagate_fused(c, 0, m->x_full, nullptr);
       return bwd_propagate(c, 0, m->x_full);
     default:
       set_error("cgcn_model_phase: unknown phase %d", kind);

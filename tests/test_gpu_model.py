@@ -659,15 +659,12 @@ def test_three_epoch_trajectory_on_a_chr22_sized_graph_keeps_per_label_auroc_aup
             assert abs(average_precision_score(t[:, c], pv[:, c].numpy()) - average_precision_score(t[:, c], pv64[:, c].numpy())) <= 1e-4, c
 
 
-@pytest.mark.parametrize("env", [{"CGCN_BWD_UNFUSED": "1"}, {"CGCN_FUSED_EPI": "8"},
-                                 {"CGCN_LAYER_MODE": "stream", "CGCN_FUSED_HEAD": "1"},
-                                 {"CGCN_LAYER_MODE": "unfused"}, {"CGCN_FUSED_GW": "8"}],
-                         ids=["bwd_unfused", "epi8", "stream_head", "unfused", "gw8"])
+@pytest.mark.parametrize("env", [{"CGCN_NO_FUSED": "1"}], ids=["unfused"])
 def test_alternative_kernel_paths_keep_parity(env):
-    """The library picks its layer kernels once per process (static switches: all-in-one gather kernel, SpMM + streamed
-    contraction kernel, the three-kernel path, the fused backward twin, the fused head, 8 epilogue / 8 gather warps).  The
-    default is whatever measured fastest; the others must stay correct: the model parity tests re-run in a subprocess
-    under each setting."""
+    """The library runs each layer either as the all-in-one fused kernel (the default at Hi-C degrees) or as three
+    kernels (SpMM, row-panel contraction, gate kernel: d != 128, weighted graphs, the FFMA contractions, mean degree
+    above 24).  CGCN_NO_FUSED, read once per process, forces the three kernels on graphs that would take the fused
+    kernel: the model parity tests re-run in a subprocess under it."""
     import subprocess
     import sys
     e = dict(os.environ)
