@@ -8,7 +8,6 @@
 // SpMM-free and lets the first layer skip its backward SpMM when nobody needs d loss / d x_in.
 #include <cstdarg>
 #include <cstdlib>
-#include <cstring>
 
 #include "common.cuh"
 #include "fused_layer.cuh"
@@ -39,7 +38,6 @@ bool tc_gram_supported(int64_t lda, int64_t ldb, int ka, int nb, const void* A, 
 size_t tc_workspace_bytes();
 
 int rowwise_max_grid();
-int bce_grid();
 int bce_launch(const float* out, const float* target, const uint32_t* target_bits, int n, int C, int S, int ld, float* probs,
                float* loss_sum, float* out_grad, float* partial, int64_t n_total, cudaStream_t stream);
 int colsum_launch(const float* X, int64_t rows, int cols, int ld, float* dst, float* partial, cudaStream_t stream);
@@ -99,19 +97,13 @@ int sm_count() {
 }
 
 // ---- dense dispatch
-static thread_local int tls_rp_ordinal = 0, tls_gr_ordinal = 0;   // developer aid (CGCN_TC_MASK_RP / _GR bitmasks)
 // one <= 128 x 128 block of the weight operand; B (with leading dimension ldb) already points at the block
 static int gemm_rowpanel_block(const float* A, int64_t lda, const float* B, int b_transposed, int64_t ldb, const float* bias, float* C,
                                int64_t ldc, int64_t m, int n, int k, const int32_t* rowscale_rowptr, const float* rowscale_inv,
                                int rowscale_group, int accumulate, int impl, void* ws, size_t ws_bytes, cudaStream_t stream,
                                const void* ready_image) {
-  static const char* dis = getenv("CGCN_TC_DISABLE");          // developer aid: "rowpanel", "gram" or "rowscale"
-  bool tc_ok = tc_rowpanel_supported(lda, ldc, n, k, A, C) &&
-               (ready_image != nullptr || (ws != nullptr && ws_bytes >= tc_workspace_bytes()));
-  if (dis && (strstr(dis, "rowpanel") || (strstr(dis, "rowscale") && rowscale_rowptr) || (strstr(dis, "head") && (n != 128 || k != 128)))) tc_ok = false;
-  static const char* mask_s = getenv("CGCN_TC_MASK_RP");
-  if (mask_s && !((atoi(mask_s) >> tls_rp_ordinal) & 1)) tc_ok = false;
-  ++tls_rp_ordinal;
+  const bool tc_ok = tc_rowpanel_supported(lda, ldc, n, k, A, C) &&
+                     (ready_image != nullptr || (ws != nullptr && ws_bytes >= tc_workspace_bytes()));
   if (impl == 2 && !tc_ok) {
     set_error("cgcn_gemm_rowpanel: tcgen05 path needs 16-byte aligned rows of a multiple of 4 floats and a workspace");
     return CGCN_ERR_INVALID;
@@ -149,12 +141,7 @@ int gemm_rowpanel_dispatch(const float* A, int64_t lda, const float* B, int b_tr
 
 static int gemm_gram_block(const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc, int64_t m,
                            int ka, int nb, int accumulate, int impl, void* ws, size_t ws_bytes, cudaStream_t stream) {
-  static const char* dis = getenv("CGCN_TC_DISABLE");
-  bool tc_ok = tc_gram_supported(lda, ldb, ka, nb, A, B);
-  if (dis && (strstr(dis, "gram") || (strstr(dis, "head") && (ka != 128 || nb != 128)))) tc_ok = false;
-  static const char* mask_s = getenv("CGCN_TC_MASK_GR");
-  if (mask_s && !((atoi(mask_s) >> tls_gr_ordinal) & 1)) tc_ok = false;
-  ++tls_gr_ordinal;
+  const bool tc_ok = tc_gram_supported(lda, ldb, ka, nb, A, B);
   if (impl == 2 && !tc_ok) {
     set_error("cgcn_gemm_gram: tcgen05 path needs 16-byte aligned rows of a multiple of 4 floats");
     return CGCN_ERR_INVALID;
@@ -316,39 +303,15 @@ struct Ctx {
   WsLayout lay;
   cudaStream_t st;
   int n, d, S, C, L, W;
+  int ldo;                          // leading dimension of out / out_grad
   int64_t M, n_total;
   bool dist;
+  bool images;                      // tcgen05 weight images prepared once per pass
+  bool fused;                       // fused layer kernels instead of SpMM + contraction + gate kernel
   float* ws;
   void* tcws;
   unsigned long long drop_off;      // float4 offset of the first local row in the global panel
 };
-
-static Ctx make_ctx(const cgcn_model* m) {
-  Ctx c;
-  c.m = m;
-  c.st = static_cast<cudaStream_t>(m->stream);
-  c.n = m->graph.n; c.d = m->d; c.S = m->strands; c.C = m->nclass; c.L = m->layers;
-  c.W = c.S * c.d;
-  c.M = static_cast<int64_t>(c.n) * c.S;
-  c.dist = m->n_total > 0;
-  c.n_total = c.dist ? m->n_total : c.n;
-  c.lay = make_layout(c.n, c.d, c.C, c.L, c.S);
-  c.ws = m->workspace;
-  c.tcws = c.ws + c.lay.tc;
-  c.drop_off = c.dist ? static_cast<unsigned long long>(m->row_begin) * c.W / 4 : 0ull;
-  return c;
-}
-
-// dropout site ids (cgcn_dropout_mask): 0 = after layer 1, 1 = after BatchNorm, l + 1 = after layer l + 1 (l >= 1)
-static int layer_drop_site(int l) { return l == 0 ? 0 : l + 1; }
-
-// Weight images of the tcgen05 contractions, one launch per pass (the weights change only at the optimiser step).
-static bool use_images(const cgcn_model* m) {
-  static const bool off = getenv("CGCN_NO_IMAGES") != nullptr;      // developer aid: per-contraction preparation
-  return m->gemm_impl != 1 && !off && m->d == 128;      // wider models prepare each 128 x 128 weight block in place
-}
-static const void* fwd_image(const Ctx& c, int i) { return use_images(c.m) ? c.ws + c.lay.img_fwd[i] : nullptr; }
-static const void* bwd_image(const Ctx& c, int i) { return use_images(c.m) ? c.ws + c.lay.img_bwd[i] : nullptr; }
 
 // The fused layer kernels (fused_layer.cu): one launch per layer and direction instead of SpMM + contraction + gate
 // kernel.  In this mode the saved `ax` panels hold the UN-normalised neighbour sums and the `dy` panels hold
@@ -358,16 +321,43 @@ static const void* bwd_image(const Ctx& c, int i) { return use_images(c.m) ? c.w
 // SM against the SpMM's ~320, so once the gather dominates (mean degree 51: fused 6.5 ms per layer vs SpMM 2.15 + 0.6 +
 // 0.9) the three kernels win: graphs with more than FUSED_MAX_DEGREE stored entries per row on average use them.
 constexpr int64_t FUSED_MAX_DEGREE = 24;
-static bool use_fused(const cgcn_model* m) {
+static bool use_fused(const cgcn_model* m, bool images) {
   static const bool off = getenv("CGCN_NO_FUSED") != nullptr;       // developer aid / A-B measurements
-  if (off || !use_images(m) || !fused_layer_supported(m->d, &m->graph)) return false;
+  if (off || !images || !fused_layer_supported(m->d, &m->graph)) return false;
   const int64_t nnz = m->graph.nnz, n = m->graph.n > 0 ? m->graph.n : 1;
   return nnz <= FUSED_MAX_DEGREE * n;
 }
 
+static Ctx make_ctx(const cgcn_model* m) {
+  Ctx c;
+  c.m = m;
+  c.st = static_cast<cudaStream_t>(m->stream);
+  c.n = m->graph.n; c.d = m->d; c.S = m->strands; c.C = m->nclass; c.L = m->layers;
+  c.W = c.S * c.d;
+  c.ldo = m->out_ld > 0 ? m->out_ld : c.C;
+  c.M = static_cast<int64_t>(c.n) * c.S;
+  c.dist = m->n_total > 0;
+  c.n_total = c.dist ? m->n_total : c.n;
+  c.lay = make_layout(c.n, c.d, c.C, c.L, c.S);
+  c.ws = m->workspace;
+  c.tcws = c.ws + c.lay.tc;
+  c.drop_off = c.dist ? static_cast<unsigned long long>(m->row_begin) * c.W / 4 : 0ull;
+  // Weight images of the tcgen05 contractions, one launch per pass (the weights change only at the optimiser step).
+  // Wider models prepare each 128 x 128 weight block in place.
+  c.images = m->gemm_impl != 1 && c.d == 128;
+  c.fused = use_fused(m, c.images);
+  return c;
+}
+
+// dropout site ids (cgcn_dropout_mask): 0 = after layer 1, 1 = after BatchNorm, l + 1 = after layer l + 1 (l >= 1)
+static int layer_drop_site(int l) { return l == 0 ? 0 : l + 1; }
+
+static const void* fwd_image(const Ctx& c, int i) { return c.images ? c.ws + c.lay.img_fwd[i] : nullptr; }
+static const void* bwd_image(const Ctx& c, int i) { return c.images ? c.ws + c.lay.img_bwd[i] : nullptr; }
+
 static int prep_fwd_images(const Ctx& c) {
   pdl_plain_next(c.st);              // first kernel of a pass: ordinary stream order against whatever ran before
-  if (!use_images(c.m)) return CGCN_OK;
+  if (!c.images) return CGCN_OK;
   TcImageSpec sp[ML + 1];
   int k = 0;
   for (int l = 0; l < c.L; ++l) sp[k++] = TcImageSpec{c.m->params.gc_w[l], 0, c.d, c.d, c.ws + c.lay.img_fwd[l]};
@@ -375,7 +365,7 @@ static int prep_fwd_images(const Ctx& c) {
   return tc_prep_images(sp, k, c.st);
 }
 static int prep_bwd_images(const Ctx& c) {
-  if (!use_images(c.m)) return CGCN_OK;
+  if (!c.images) return CGCN_OK;
   TcImageSpec sp[ML + 1];
   int k = 0;
   sp[k++] = TcImageSpec{c.m->params.out_w, 0, c.d, c.C, c.ws + c.lay.img_bwd[0]};
@@ -409,7 +399,7 @@ static int fwd_layer(const Ctx& c, int l, const float* gather_src) {
   const float* xin = (l == 0) ? m->x_in : ws + lay.xo[l - 1];
   const bool last = (l == c.L - 1);
   int grid = 0;
-  if (use_fused(m)) {
+  if (c.fused) {
     // gather -> (A_hat x) W + b -> tanh -> gate -> blend -> dropout (-> BatchNorm column sums) in one kernel
     fl::Args a{};
     a.rowptr = m->graph.rowptr;
@@ -481,13 +471,11 @@ static int fwd_head(const Ctx& c) {
   b.drop = make_dropout(m->dropout_p, m->seed, m->step, 1, m->training, c.drop_off);
   CGCN_TRY(bn_apply_launch(b, c.st));
   // out = hb Wout^T + bout                           (models/ChromeModels.py:51)
-  const int ldo = m->out_ld > 0 ? m->out_ld : c.C;
-  return gemm_rowpanel_dispatch(ws + lay.hb, c.d, m->params.out_w, 1, m->params.out_b, m->out, ldo, c.M, c.C, c.d, nullptr, nullptr,
+  return gemm_rowpanel_dispatch(ws + lay.hb, c.d, m->params.out_w, 1, m->params.out_b, m->out, c.ldo, c.M, c.C, c.d, nullptr, nullptr,
                                 1, m->gemm_impl, c.tcws, lay.tc_bytes, c.st, fwd_image(c, c.L));
 }
 
 static int model_forward(const cgcn_model* m) {
-  tls_rp_ordinal = tls_gr_ordinal = 0;
   CGCN_TRY(validate(m, false));
   CGCN_REQUIRE(m->n_total <= 0, "cgcn_model_forward: row-partitioned graphs (n_total > 0) run through cgcn_model_phase");
   const Ctx c = make_ctx(m);
@@ -497,9 +485,9 @@ static int model_forward(const cgcn_model* m) {
 }
 
 // ---- backward stages.  Scratch panels: one dy per layer (never rewritten while the side stream's gram kernel reads
-// it) and three rotating ones.  Layer l reads the gradient entering its gate stage from src(l), writes dy_l and
-// dxd (dC), overwrites src(l) with t_l = D^-1 (dy_l W_l^T), and the SpMM writes dx = dC + P t_l into the other
-// rotating panel, which is src(l-1).
+// it) and three rotating ones.  On the three-kernel path layer l reads the gradient entering its gate stage from
+// src(l), writes dy_l and dxd (dC), overwrites src(l) with t_l = D^-1 (dy_l W_l^T), and the SpMM writes
+// dx = dC + P t_l into the other rotating panel, which is src(l-1).
 struct Fork {
   SideStream* side;
   cudaStream_t st, ss;
@@ -522,9 +510,10 @@ struct Fork {
   }
 };
 
-static int make_fork(const Ctx& c, Fork* f) {
+// serial: the side-stream work runs in order on the caller's stream
+static int make_fork(const Ctx& c, bool serial, Fork* f) {
   static const bool no_side = getenv("CGCN_NO_SIDE_STREAM") != nullptr;   // developer aid
-  f->serial = no_side;
+  f->serial = serial || no_side;
   f->st = c.st;
   f->side = nullptr;
   f->ss = c.st;
@@ -545,13 +534,12 @@ static int bwd_head(const Ctx& c, Fork& f) {
   float* ws = c.ws;
   float* dhb = bwd_src(c, c.L - 1);
   void* gram_ws = ws + lay.gram;               // used by the side stream only
-  const int ldo = m->out_ld > 0 ? m->out_ld : c.C;
   CGCN_TRY(prep_bwd_images(c));
   CGCN_TRY(f.fork());
-  CGCN_TRY(gemm_gram_dispatch(m->out_grad, ldo, ws + lay.hb, c.d, m->grads.out_w, c.d, c.M, c.C, c.d, 0, m->gemm_impl, gram_ws,
+  CGCN_TRY(gemm_gram_dispatch(m->out_grad, c.ldo, ws + lay.hb, c.d, m->grads.out_w, c.d, c.M, c.C, c.d, 0, m->gemm_impl, gram_ws,
                               lay.gram_bytes, f.ss));
-  CGCN_TRY(colsum_launch(m->out_grad, c.M, c.C, ldo, m->grads.out_b, ws + lay.partial_side, f.ss));
-  CGCN_TRY(gemm_rowpanel_dispatch(m->out_grad, ldo, m->params.out_w, 0, nullptr, dhb, c.d, c.M, c.d, c.C, nullptr, nullptr, 1,
+  CGCN_TRY(colsum_launch(m->out_grad, c.M, c.C, c.ldo, m->grads.out_b, ws + lay.partial_side, f.ss));
+  CGCN_TRY(gemm_rowpanel_dispatch(m->out_grad, c.ldo, m->params.out_w, 0, nullptr, dhb, c.d, c.M, c.d, c.C, nullptr, nullptr, 1,
                                   m->gemm_impl, c.tcws, lay.tc_bytes, c.st, bwd_image(c, 0)));
   BnBwdReduceArgs r{};
   r.dhb = dhb;
@@ -568,27 +556,27 @@ static int bwd_head(const Ctx& c, Fork& f) {
                                 m->grads.bn_w, m->grads.bn_b, nullptr, c.dist ? m->bn_sums : nullptr, c.st);
 }
 
-// gradient entering layer l_from - 1 (or x_in_grad) = dxd + P t, with t gathered from `t_gather` (layer l_from's t, or
-// its all-gathered copy)
-static int bwd_propagate(const Ctx& c, int l_from, const float* t_gather) {
-  float* dx = (l_from == 0) ? c.m->x_in_grad : bwd_other(c, l_from);
-  if (c.dist && c.m->peer != nullptr) return spmm_peer_launch(&c.m->graph, c.m->peer, dx, c.W, 0, c.ws + c.lay.dC, c.st);
-  return spmm_launch(&c.m->graph, t_gather, dx, c.W, 0, c.ws + c.lay.dC, c.st);
-}
-
-// ---- fused backward (use_fused): the gather comes first, A_hat^T G W^T = (P (D^-1 G)) W^T.
-// Gradient entering layer l_from - 1 from layer l_from: one kernel gathers u = P dys_{l_from}, contracts u W^T, adds
-// (1-g) dh (dC) and, for l_from > 0, runs the whole gate / tanh backward of layer l_from - 1 in its epilogue (writes
-// dys_{l_from-1}, dC, the column partials; *parts = partial rows written).  l_from == 0: d loss / d x_in.
-static int bwd_propagate_fused(const Ctx& c, int l_from, const float* gather_src, int* parts) {
+// Gradient entering layer l_from - 1 (or x_in_grad) from layer l_from; `gather` is the panel the next propagate reads
+// (bwd_layer's *t_out, or its all-gathered copy).
+// Three kernels: dx = dxd + P t, with t = D^-1 (dy W^T), into the other rotating panel.
+// Fused: the gather comes first, A_hat^T G W^T = (P (D^-1 G)) W^T.  One kernel gathers u = P dys_{l_from}, contracts
+// u W^T, adds (1-g) dh (dC) and, for l_from > 0, runs the whole gate / tanh backward of layer l_from - 1 in its epilogue
+// (writes dys_{l_from-1}, dC, the column partials; *parts = partial rows written).  l_from == 0: d loss / d x_in.
+// `parts` may be NULL.
+static int bwd_propagate(const Ctx& c, int l_from, const float* gather, int* parts) {
   const cgcn_model* m = c.m;
   const WsLayout& lay = c.lay;
   float* ws = c.ws;
+  if (!c.fused) {
+    float* dx = (l_from == 0) ? m->x_in_grad : bwd_other(c, l_from);
+    if (c.dist && m->peer != nullptr) return spmm_peer_launch(&m->graph, m->peer, dx, c.W, 0, ws + lay.dC, c.st);
+    return spmm_launch(&m->graph, gather, dx, c.W, 0, ws + lay.dC, c.st);
+  }
   fl::Args a{};
   a.rowptr = m->graph.rowptr;
   a.colidx = m->graph.colidx;
   a.n = c.n;
-  a.gsrc = gather_src;
+  a.gsrc = gather;
   if (c.dist && m->peer != nullptr) CGCN_TRY(fused_layer_set_peer(&a, m->peer, c.n));
   a.w = m->params.gc_w[l_from];
   a.w_transposed = 1;
@@ -611,24 +599,26 @@ static int bwd_propagate_fused(const Ctx& c, int l_from, const float* gather_src
   return fused_layer_launch(a, c.S, fl::BWD_MID, parts, c.st);
 }
 
-// Layer l in fused mode.  Head layer: BatchNorm / ReLU / gate backward as a row-wise kernel that stores D^-1 dy.
-// Other layers: their gate stage already ran in the epilogue of bwd_propagate_fused(l + 1) (`parts` partial rows).
-// Then, on the side stream: bias / gate gradients from the partials and d W = ax^T dys.  *t_out = the panel the next
-// propagate gathers (NULL if the chain stops here).
-static int bwd_layer_fused(const Ctx& c, Fork& f, int l, int parts, const float** t_out) {
+// Gate stage of layer l, its weight gradients (side stream) and the panel the next propagate gathers.
+// The gate stage is a row-wise kernel for the head layer and on the three-kernel path; in fused mode it stores
+// D^-1 dy, and the gate stage of every other layer already ran in the epilogue of bwd_propagate(l + 1) (`parts`
+// partial rows).  *t_out = dy in fused mode, else t = D^-1 (dy W^T) in the panel that held src(l); NULL if the chain
+// stops here.
+static int bwd_layer(const Ctx& c, Fork& f, int l, int parts, const float** t_out) {
   const cgcn_model* m = c.m;
   const WsLayout& lay = c.lay;
   float* ws = c.ws;
   const bool head = (l == c.L - 1);
   const bool need_dx = (l > 0) || m->need_input_grad;
+  float* src = bwd_src(c, l);
   float* dy = ws + lay.dy[l];
   *t_out = nullptr;
-  if (head) {
-    if (c.dist)                      // c1, c2 from the all-reduced BatchNorm backward sums
-      CGCN_TRY(bn_bwd_finalize_launch(ws + lay.partial, 0, c.n_total, c.S, c.d, m->training, ws + lay.bn_c1, ws + lay.bn_c2, nullptr,
-                                      nullptr, m->bn_sums, nullptr, c.st));
+  if (head && c.dist)                // c1, c2 from the all-reduced BatchNorm backward sums
+    CGCN_TRY(bn_bwd_finalize_launch(ws + lay.partial, 0, c.n_total, c.S, c.d, m->training, ws + lay.bn_c1, ws + lay.bn_c2, nullptr,
+                                    nullptr, m->bn_sums, nullptr, c.st));
+  if (head || !c.fused) {
     GateBwdArgs a{};
-    a.dsrc = bwd_src(c, l);
+    a.dsrc = src;
     a.h = ws + lay.xo[l];
     a.mean = ws + lay.bn_mean;
     a.rstd = ws + lay.bn_rstd;
@@ -643,57 +633,20 @@ static int bwd_layer_fused(const Ctx& c, Fork& f, int l, int parts, const float*
     a.dxd = need_dx ? ws + lay.dC : nullptr;
     a.partial = ws + lay.partial_l[l];
     a.n = c.n;
-    a.drop = make_dropout(m->dropout_p, m->seed, m->step, 1, m->training, c.drop_off);
-    a.scale_rowptr = m->graph.rowptr;
-    CGCN_TRY(gate_bwd_launch(a, c.d, c.S, true, &parts, c.st));
+    a.drop = make_dropout(m->dropout_p, m->seed, m->step, head ? 1 : layer_drop_site(l), m->training, c.drop_off);
+    a.scale_rowptr = c.fused ? m->graph.rowptr : nullptr;
+    CGCN_TRY(gate_bwd_launch(a, c.d, c.S, head, &parts, c.st));
   }
+  // side: bias / gate gradients from the partials, d W = (A_hat x)^T dy
   CGCN_TRY(f.fork());
   CGCN_TRY(gate_bwd_finalize_launch(ws + lay.partial_l[l], parts, c.d, m->grads.gc_b[l], m->grads.gate_w[l], m->grads.gate_b[l], f.ss));
   CGCN_TRY(gemm_gram_dispatch(ws + lay.ax[l], c.d, dy, c.d, m->grads.gc_w[l], c.d, c.M, c.d, c.d, 0, m->gemm_impl, ws + lay.gram,
                               lay.gram_bytes, f.ss));
-  if (need_dx) *t_out = dy;
-  return CGCN_OK;
-}
-
-// gate stage of layer l, its weight gradients (side stream) and, if anything upstream needs it, t = D^-1 (dy W^T).
-// Returns in *t_out the panel holding t (NULL if the chain stops here).
-static int bwd_layer(const Ctx& c, Fork& f, int l, const float** t_out) {
-  const cgcn_model* m = c.m;
-  const WsLayout& lay = c.lay;
-  float* ws = c.ws;
-  const bool head = (l == c.L - 1);
-  const bool need_dx = (l > 0) || m->need_input_grad;
-  float* src = bwd_src(c, l);
-  float* dy = ws + lay.dy[l];
-  *t_out = nullptr;
-  if (head && c.dist)                // c1, c2 from the all-reduced BatchNorm backward sums
-    CGCN_TRY(bn_bwd_finalize_launch(ws + lay.partial, 0, c.n_total, c.S, c.d, m->training, ws + lay.bn_c1, ws + lay.bn_c2, nullptr,
-                                    nullptr, m->bn_sums, nullptr, c.st));
-  GateBwdArgs a{};
-  a.dsrc = src;
-  a.h = ws + lay.xo[l];
-  a.mean = ws + lay.bn_mean;
-  a.rstd = ws + lay.bn_rstd;
-  a.gamma = m->params.bn_w;
-  a.c1 = ws + lay.bn_c1;
-  a.c2 = ws + lay.bn_c2;
-  a.z = ws + lay.z[l];
-  a.x = (l == 0) ? m->x_in : ws + lay.xo[l - 1];
-  a.g = m->gate[l];
-  a.wg = m->params.gate_w[l];
-  a.dy = dy;
-  a.dxd = need_dx ? ws + lay.dC : nullptr;
-  a.partial = ws + lay.partial_l[l];
-  a.n = c.n;
-  a.drop = make_dropout(m->dropout_p, m->seed, m->step, head ? 1 : layer_drop_site(l), m->training, c.drop_off);
-  int grid = 0;
-  CGCN_TRY(gate_bwd_launch(a, c.d, c.S, head, &grid, c.st));
-  // side: bias / gate gradients from the partials, d W = (A_hat x)^T dy
-  CGCN_TRY(f.fork());
-  CGCN_TRY(gate_bwd_finalize_launch(ws + lay.partial_l[l], grid, c.d, m->grads.gc_b[l], m->grads.gate_w[l], m->grads.gate_b[l], f.ss));
-  CGCN_TRY(gemm_gram_dispatch(ws + lay.ax[l], c.d, dy, c.d, m->grads.gc_w[l], c.d, c.M, c.d, c.d, 0, m->gemm_impl, ws + lay.gram,
-                              lay.gram_bytes, f.ss));
   if (!need_dx) return CGCN_OK;
+  if (c.fused) {
+    *t_out = dy;
+    return CGCN_OK;
+  }
   // main: t = D^-1 (dy W^T) -> the panel that held `src`
   CGCN_TRY(gemm_rowpanel_dispatch(dy, c.d, m->params.gc_w[l], 1, nullptr, src, c.d, c.M, c.d, c.d, m->graph.rowptr,
                                   m->graph.row_inv, c.S, m->gemm_impl, c.tcws, lay.tc_bytes, c.st, bwd_image(c, 1 + l)));
@@ -706,23 +659,14 @@ static int model_backward(const cgcn_model* m) {
   CGCN_REQUIRE(m->n_total <= 0, "cgcn_model_backward: row-partitioned graphs (n_total > 0) run through cgcn_model_phase");
   const Ctx c = make_ctx(m);
   Fork f;
-  CGCN_TRY(make_fork(c, &f));
+  CGCN_TRY(make_fork(c, false, &f));
   CGCN_TRY(bwd_head(c, f));
-  if (use_fused(m)) {
-    int parts = 0;
-    for (int l = c.L - 1; l >= 0; --l) {
-      const float* t = nullptr;
-      CGCN_TRY(bwd_layer_fused(c, f, l, parts, &t));
-      if (t == nullptr) break;
-      CGCN_TRY(bwd_propagate_fused(c, l, t, &parts));      // also the gate stage of layer l - 1
-    }
-    return f.join();
-  }
+  int parts = 0;
   for (int l = c.L - 1; l >= 0; --l) {
     const float* t = nullptr;
-    CGCN_TRY(bwd_layer(c, f, l, &t));
+    CGCN_TRY(bwd_layer(c, f, l, parts, &t));
     if (t == nullptr) break;
-    CGCN_TRY(bwd_propagate(c, l, t));
+    CGCN_TRY(bwd_propagate(c, l, t, &parts));
   }
   return f.join();
 }
@@ -737,16 +681,12 @@ static int model_phase(const cgcn_model* m, int kind, int layer, const float** p
   CGCN_REQUIRE(layer >= 0 && layer < m->layers, "cgcn_model_phase: layer %d", layer);
   const Ctx c = make_ctx(m);
   Fork f;
-  f.serial = true;                   // stage by stage: everything on the caller's stream
-  f.st = f.ss = c.st;
-  f.side = nullptr;
+  CGCN_TRY(make_fork(c, true, &f));  // stage by stage: everything on the caller's stream
   const float* t = nullptr;
+  int parts = 0;
   switch (kind) {
     case CGCN_PHASE_FWD_LAYER:       // x_full holds the gathered input of `layer`
-      if (layer == 0) {
-        tls_rp_ordinal = tls_gr_ordinal = 0;
-        CGCN_TRY(prep_fwd_images(c));
-      }
+      if (layer == 0) CGCN_TRY(prep_fwd_images(c));
       CGCN_TRY(fwd_layer(c, layer, m->x_full));
       if (publish && layer + 1 < c.L) *publish = c.ws + c.lay.xo[layer];
       return CGCN_OK;
@@ -755,20 +695,13 @@ static int model_phase(const cgcn_model* m, int kind, int layer, const float** p
     case CGCN_PHASE_BWD_HEAD:
       return bwd_head(c, f);
     case CGCN_PHASE_BWD_LAYER:       // layer == L-1: bn_sums all-reduced ; else: x_full holds the gathered t of layer+1
-      if (use_fused(m)) {
-        int parts = 0;
-        if (layer < c.L - 1) CGCN_TRY(bwd_propagate_fused(c, layer + 1, m->x_full, &parts));
-        CGCN_TRY(bwd_layer_fused(c, f, layer, parts, &t));
-      } else {
-        if (layer < c.L - 1) CGCN_TRY(bwd_propagate(c, layer + 1, m->x_full));
-        CGCN_TRY(bwd_layer(c, f, layer, &t));
-      }
+      if (layer < c.L - 1) CGCN_TRY(bwd_propagate(c, layer + 1, m->x_full, &parts));
+      CGCN_TRY(bwd_layer(c, f, layer, parts, &t));
       if (publish) *publish = t;
       return CGCN_OK;
     case CGCN_PHASE_BWD_INPUT:       // x_full holds the gathered t of layer 0
       CGCN_REQUIRE(m->need_input_grad && m->x_in_grad, "cgcn_model_phase: BWD_INPUT without need_input_grad");
-      if (use_fused(m)) return bwd_propagate_fused(c, 0, m->x_full, nullptr);
-      return bwd_propagate(c, 0, m->x_full);
+      return bwd_propagate(c, 0, m->x_full, nullptr);
     default:
       set_error("cgcn_model_phase: unknown phase %d", kind);
       return CGCN_ERR_INVALID;
@@ -894,9 +827,9 @@ static int train_step(const cgcn_model* m, const float* target, const uint32_t* 
                       float* out_grad_scratch) {
   CGCN_REQUIRE(m && (target || target_bits) && loss_sum_out && out_grad_scratch, "cgcn_train_step: null argument");
   CGCN_TRY(model_forward(m));
-  const WsLayout lay = make_layout(m->graph.n, m->d, m->nclass, m->layers, m->strands);
-  CGCN_TRY(bce_launch(m->out, target, target_bits, m->graph.n, m->nclass, m->strands, m->out_ld > 0 ? m->out_ld : m->nclass, probs,
-                      loss_sum_out, out_grad_scratch, m->workspace + lay.partial, 0, static_cast<cudaStream_t>(m->stream)));
+  const Ctx c = make_ctx(m);
+  CGCN_TRY(bce_launch(m->out, target, target_bits, c.n, c.C, c.S, c.ldo, probs, loss_sum_out, out_grad_scratch, c.ws + c.lay.partial, 0,
+                      c.st));
   cgcn_model mb = *m;
   mb.out_grad = out_grad_scratch;
   return model_backward(&mb);

@@ -843,11 +843,6 @@ int gate_bwd_finalize_launch(const float* partial, int grid, int d, float* db, f
   return check_launch("col_finalize_kernel");
 }
 
-size_t colsum_workspace_floats(int64_t rows) {
-  (void)rows;
-  return static_cast<size_t>(sm_count()) * 8 * 128;
-}
-
 int colsum_launch(const float* X, int64_t rows, int cols, int ld, float* dst, float* partial, cudaStream_t stream) {
   CGCN_REQUIRE(cols >= 1 && cols <= 128, "colsum: cols=%d", cols);
   const int64_t max_parts = static_cast<int64_t>(sm_count()) * 8;
