@@ -790,6 +790,7 @@ extern "C" int cgcn_gcn_layer_bwd(const cgcn_graph* g, int32_t strands, const fl
                                   cgcn_stream_t stream) {
   CGCN_REQUIRE(g && dys_gather && dxd && W, "cgcn_gcn_layer_bwd: null argument");
   CGCN_REQUIRE(fused_layer_supported(128, g), "cgcn_gcn_layer_bwd: pattern graphs only (no value array)");
+  CGCN_REQUIRE(dropout_p >= 0.f && dropout_p < 1.f, "cgcn_gcn_layer_bwd: dropout_p=%f", dropout_p);
   fl::Args a{};
   a.rowptr = g->rowptr;
   a.colidx = g->colidx;

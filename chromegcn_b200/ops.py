@@ -80,21 +80,46 @@ def spmm_peer(graph: HiCGraph, blocks: Sequence[torch.Tensor], rank: int, mean: 
     return out
 
 
+def _out(t: Optional[torch.Tensor], shape, device, more_rows: bool = False) -> torch.Tensor:
+    """Output buffer of a kernel: a new tensor, or the caller's, which the kernel writes in place (so it is checked, not
+    copied like `_f32c` inputs; a view into a larger buffer is fine).  `more_rows`: the caller's tensor may have more
+    rows than `shape` (per-CTA partials)."""
+    if t is None:
+        return torch.empty(*shape, dtype=torch.float32, device=device)
+    if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.data_ptr() % 16 != 0:
+        raise _lib.ChromeGCNNativeError("output tensors must be contiguous, 16-byte aligned CUDA float32")
+    rows_ok = t.shape[0] >= shape[0] if more_rows else t.shape[0] == shape[0]
+    if t.dim() != len(shape) or tuple(t.shape[1:]) != tuple(shape[1:]) or not rows_ok:
+        raise _lib.ChromeGCNNativeError("output tensor of shape %s, need %s" % (tuple(t.shape), tuple(shape)))
+    return t
+
+
+def _max_layer_parts(n: int, strands: int, device) -> int:
+    """Upper bound of the fused layer kernel's CTA count (= partial rows it writes): one CTA per 64-row panel tile, at
+    most one per SM (fused_layer_grid)."""
+    tiles = (n * strands + 63) // 64
+    return max(1, min(tiles, torch.cuda.get_device_properties(device).multi_processor_count))
+
+
 def gcn_layer_fwd(graph: HiCGraph, x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, gate_w: Optional[torch.Tensor],
                   gate_b: Optional[torch.Tensor], gate_off: bool = False, dropout_p: float = 0.0, seed: int = 0, step: int = 0,
-                  site: int = 0, with_stats: bool = False, x_gather: Optional[torch.Tensor] = None):
+                  site: int = 0, with_stats: bool = False, x_gather: Optional[torch.Tensor] = None,
+                  x_out: Optional[torch.Tensor] = None, z_out: Optional[torch.Tensor] = None,
+                  gate_out: Optional[torch.Tensor] = None, sx_out: Optional[torch.Tensor] = None,
+                  stats_out: Optional[torch.Tensor] = None):
     """One gated GCN layer (models/ChromeModels.py:37-40) as one fused kernel (cgcn_gcn_layer_fwd).  `x` is
     `[n, 128]` or the strand-interleaved `[n, S, 128]`.  Returns `(x_out, z, gate, sx, stats)`; `stats` is the
-    `[parts, 2*S*128]` per-CTA column sums of relu(x_out), relu(x_out)^2 (None unless `with_stats`)."""
+    `[parts, 2*S*128]` per-CTA column sums of relu(x_out), relu(x_out)^2 (None unless `with_stats`).  The `*_out`
+    tensors, when given, receive the results (`stats_out`: at least as many rows as the kernel has CTAs)."""
     lib = _lib.load()
     x = _f32c(x)
     n = graph.n
     S = x.shape[1] if x.dim() == 3 else 1
     dev = x.device
     xg = x if x_gather is None else _f32c(x_gather)
-    sx, z, xo = torch.empty_like(x), torch.empty_like(x), torch.empty_like(x)
-    gate = torch.empty(n, S, dtype=torch.float32, device=dev)
-    stats = torch.zeros(512, 2 * S * 128, dtype=torch.float32, device=dev) if with_stats else None
+    sx, z, xo = _out(sx_out, x.shape, dev), _out(z_out, x.shape, dev), _out(x_out, x.shape, dev)
+    gate = _out(gate_out, (n, S), dev)
+    stats = _out(stats_out, (_max_layer_parts(n, S, dev), 2 * S * 128), dev, more_rows=True) if with_stats else None
     parts = C.c_int32(0)
     gs = graph.c_struct()
     with torch.cuda.device(dev):
@@ -105,6 +130,50 @@ def gcn_layer_fwd(graph: HiCGraph, x: torch.Tensor, weight: torch.Tensor, bias: 
                                           gate.data_ptr(), _lib.ptr(stats), C.byref(parts), _lib.current_stream()),
                    "cgcn_gcn_layer_fwd")
     return xo, z, gate, sx, (stats[: parts.value] if with_stats else None)
+
+
+_NEW = object()          # gcn_layer_bwd(dxd_out=...) default: a new panel
+
+
+def gcn_layer_bwd(graph: HiCGraph, dys_gather: torch.Tensor, dxd: torch.Tensor, weight: torch.Tensor,
+                  z_prev: Optional[torch.Tensor] = None, x_prev: Optional[torch.Tensor] = None,
+                  g_prev: Optional[torch.Tensor] = None, wg_prev: Optional[torch.Tensor] = None, gate_off: bool = False,
+                  dropout_p: float = 0.0, seed: int = 0, step: int = 0, site_prev: int = 0,
+                  dys_out: Optional[torch.Tensor] = None, dxd_out=_NEW, dx_out: Optional[torch.Tensor] = None,
+                  partial: Optional[torch.Tensor] = None):
+    """The backward twin of `gcn_layer_fwd` (cgcn_gcn_layer_bwd): `dys_gather` is D^-1 dy of this layer (the panel the
+    column indices address), `dxd` its (1-g) dh, `weight` its `[128 in, 128 out]` W; panels as in `gcn_layer_fwd`.
+    With the layer below (`z_prev`, `x_prev`, `g_prev` `[n, S]`, `wg_prev`; `dropout_p` / `seed` / `step` / `site_prev`
+    draw its output's keep-mask) returns `(dys_out, dxd_out, partial[:parts])`: D^-1 dy and (1-g) dh of the layer below
+    and the per-CTA column sums `d b | d w_g | d b_g` (`[parts, 260]`).  `dxd_out` may be `dxd` (updated in place) or
+    None (not written).  Without it (`z_prev` None) returns `dx_out` = d loss / d x_in.  The output tensors, when given,
+    receive the results (`partial`: at least as many rows as the kernel has CTAs)."""
+    lib = _lib.load()
+    dys_gather = _f32c(dys_gather)
+    n = graph.n
+    S = dys_gather.shape[1] if dys_gather.dim() == 3 else 1
+    dev = dys_gather.device
+    shape = dys_gather.shape
+    mid = z_prev is not None
+    if mid:
+        dys_out = _out(dys_out, shape, dev)
+        dxd_out = None if dxd_out is None else _out(None if dxd_out is _NEW else dxd_out, shape, dev)
+        partial = _out(partial, (_max_layer_parts(n, S, dev), 2 * 128 + 4), dev, more_rows=True)
+        dx_out = None
+    else:
+        dx_out = _out(dx_out, shape, dev)
+        dys_out = dxd_out = partial = None
+    dxd_in = dxd_out if dxd_out is dxd else _f32c(dxd)      # in place: the kernel reads and writes the caller's buffer
+    opt = lambda t: _lib.ptr(None if t is None else _f32c(t))
+    parts = C.c_int32(0)
+    gs = graph.c_struct()
+    with torch.cuda.device(dev):
+        _lib.check(lib.cgcn_gcn_layer_bwd(C.byref(gs), S, dys_gather.data_ptr(), dxd_in.data_ptr(), _f32c(weight).data_ptr(),
+                                          opt(z_prev), opt(x_prev), opt(g_prev), opt(wg_prev), 1 if gate_off else 0,
+                                          float(dropout_p), seed, step, site_prev, _lib.ptr(dys_out), _lib.ptr(dxd_out),
+                                          _lib.ptr(dx_out), _lib.ptr(partial), C.byref(parts), _lib.current_stream()),
+                   "cgcn_gcn_layer_bwd")
+    return (dys_out, dxd_out, partial[: parts.value]) if mid else dx_out
 
 
 def gemm_rowpanel(a: torch.Tensor, b: torch.Tensor, b_transposed: bool = False, bias: Optional[torch.Tensor] = None,

@@ -225,6 +225,7 @@ int cgcn_gcn_layer_fwd(const cgcn_graph* g, int32_t strands, const float* x_gath
  *   dz = g_prev dh + dgp wg_prev ; dy_prev = dz (1 - z_prev^2) ; dys_out = D^-1 dy_prev ; dxd_out = (1 - g_prev) dh
  *   partial[*parts_host][2*128+4]: per-CTA column sums of dy_prev | dgp z_prev | dgp   (d b, d w_g, d b_g)
  * With z_prev == NULL, dx is written to dx_out (d loss / d x_in) and nothing else.  dxd_out may be NULL or alias dxd.
+ * dropout_p must lie in [0, 1) (0: no mask), as in cgcn_gcn_layer_fwd.
  */
 int cgcn_gcn_layer_bwd(const cgcn_graph* g, int32_t strands, const float* dys_gather, const float* dxd, const float* W,
                        const float* z_prev, const float* x_prev, const float* g_prev, const float* wg_prev, int32_t gate_off,

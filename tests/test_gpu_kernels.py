@@ -6,6 +6,7 @@ Tolerances (max-norm relative, `oracle.gcn.max_rel`):
   * fp32 FFMA contractions: 2e-6 against fp64;
   * tcgen05 3xTF32 contractions: 1e-5 against fp64 (north_star budget), and reported.
 """
+import functools
 import os
 
 import numpy as np
@@ -417,16 +418,110 @@ def _elementwise_rel(got, ref, floor):
     return float(((got - ref).abs() / denom).max())
 
 
+# ------------------------------------------------------------------------------ fused layer kernel (csrc/fused_layer.cu)
+def _cdiv(a, b):
+    return -(-a // b)
+
+
+def _sms():
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def _fused_grid(n, strands, sms):
+    """Python copy of fused_layer_grid (csrc/fused_layer.cu): `(CTAs, window rows per CTA)`.  A CTA runs its rows as
+    tiles of 64 / strands window rows; the tests below pick their sizes and place their edge-case rows with it, and
+    check the kernel's CTA count against it, so a change of the rule fails them instead of moving them to another
+    regime unnoticed."""
+    grid = max(min(_cdiv(n, 64 // strands), sms), 1)
+    rows = max(_cdiv(_cdiv(n, grid), 4) * 4, 4)
+    return max(_cdiv(n, rows), 1), rows
+
+
+# "one_tile": 2777 rows are one tile per CTA on 148 SMs (44 CTAs x 64 rows with one strand, 87 x 32 with two).
+# "multi_tile": every CTA but the last runs >= 3 tiles and the last of them is partly filled: on 148 SMs, one strand
+# 31 111 rows = 147 CTAs x 212 (4 tiles, the last holding 20), two strands 15 557 = 145 x 108 (4 tiles, the last
+# holding 12).  Other SM counts scale n and take the next n with these properties.
+_ONE_TILE_N = 2777
+_MULTI_TILE_N_148 = {1: 31111, 2: 15557}
+
+
+def _layer_n(strands, size):
+    if size == "one_tile":
+        return _ONE_TILE_N
+    sms, tg = _sms(), 64 // strands
+    n0 = _MULTI_TILE_N_148[strands] * sms // 148
+    for n in range(n0, 2 * n0):
+        grid, rows = _fused_grid(n, strands, sms)
+        if grid >= 10 and rows % tg != 0 and _cdiv(rows, tg) >= 3:
+            return n
+    raise AssertionError("no multi-tile size for %d SMs" % sms)
+
+
+_HUB = 913      # stored entries of a hub row, self loop included: 29 segments of <= 32 column indices
+
+
+def _edge_case_graph(n, strands, seed=11):
+    """A near-diagonal Hi-C-like symmetric pattern (mean degree ~13 with the self loops) in which rows at positions
+    taken from the grid have exactly 1 (self loop only), 32, 33, 64, 65 (the segment and batch edges of the gather for
+    U = 3 and 6) or _HUB stored entries: at the first and last row of a CTA, at a tile's first or last row and in the
+    middle of a tile.  Edges of these rows lead to other rows only, so the counts are exact.  Returns
+    `(indptr, indices, graph)`, the CSR without the self loops the graph adds."""
+    grid, rows = _fused_grid(n, strands, _sms())
+    tg = 64 // strands
+    ntile = _cdiv(rows, tg)
+    last = (ntile - 1) * tg                      # offset of a CTA's last tile
+    cta = lambda c: c * rows
+    assert grid >= 10
+    want = {cta(1): 1, cta(3) - 1: 1,            # self loop only: first row of one CTA, last row of another
+            cta(4) - 1: _HUB,                    # hub: last row of a CTA ...
+            cta(5) + min(2, ntile - 1) * tg: _HUB,   # ... and first row of a tile inside one (its third, if it has one)
+            cta(6) + min(tg, rows) - 1: 32,      # last row of a CTA's first tile
+            cta(7) + last: 33,                   # first row of a CTA's last tile
+            cta(8) + last + 1: 64, cta(9) - 1: 65,   # inside and at the end of a CTA's last tile
+            cta(9) + 4: 32, cta(9) + 5: 33, cta(9) + 6: 64, cta(9) + 7: 65}
+    rng = np.random.default_rng(seed)
+    m = n * 6
+    i = rng.integers(0, n, m)
+    j = np.clip(i + rng.integers(1, 200, m), 0, n - 1)
+    special = np.zeros(n, dtype=bool)
+    special[list(want)] = True
+    keep = (i != j) & ~special[i] & ~special[j]
+    pi, pj = [i[keep]], [j[keep]]
+    free = np.flatnonzero(~special)
+    for r, k in want.items():
+        if k == _HUB:
+            partners = rng.choice(free, k - 1, replace=False)
+        else:                                    # the nearest ordinary rows: a near-diagonal band
+            partners = free[np.argsort(np.abs(free - r), kind="stable")[: k - 1]]
+        pi.append(np.full(k - 1, r))
+        pj.append(partners)
+    ip, ix = oadj._pairs_to_csr(n, np.concatenate(pi), np.concatenate(pj))
+    g = _graph(ip, ix)
+    deg = np.diff(g.csr_numpy()[0])
+    assert all(deg[r] == k for r, k in want.items()), {r: (k, deg[r]) for r, k in want.items()}
+    assert 10 <= g.nnz / n <= 15
+    return ip, ix, g
+
+
+_FWD_CASES = ([pytest.param(m, "one_tile", id=m) for m in ("plain", "gate_off", "dropout", "stats", "hubs")] +
+              [pytest.param(m, "multi_tile", id=m + "-multi_tile") for m in ("plain", "gate_off", "dropout", "stats")])
+
+
 @pytest.mark.parametrize("strands", [1, 2])
-@pytest.mark.parametrize("mode", ["plain", "gate_off", "dropout", "stats", "hubs"])
-def test_fused_layer_fwd_matches_fp64(strands, mode):
+@pytest.mark.parametrize("mode,size", _FWD_CASES)
+def test_fused_layer_fwd_matches_fp64(strands, mode, size):
     """cgcn_gcn_layer_fwd (one kernel: gather -> tcgen05 3xTF32 -> gate epilogue) against the layer of
     models/ChromeModels.py:37-40 + models/SubLayers.py:42-52 in fp64 torch on the same inputs; the dropout case feeds
-    the oracle the kernel's own keep-mask (cgcn_dropout_mask)."""
+    the oracle the kernel's own keep-mask (cgcn_dropout_mask).  The multi-tile cases run several tiles per CTA on the
+    edge-case graph; their stats case checks column partials accumulated over several tiles."""
     from chromegcn_b200 import ops
-    n = 2777 if mode != "hubs" else 1500                 # not a multiple of the 64-row tile; several CTAs
-    ip, ix = _random_pattern(n, 14, 11, hub=900 if mode == "hubs" else None)     # row 7 of "hubs" spans 29 segments
-    g = _graph(ip, ix)
+    if size == "multi_tile":
+        n = _layer_n(strands, size)
+        ip, ix, g = _edge_case_graph(n, strands)
+    else:
+        n = _ONE_TILE_N if mode != "hubs" else 1500      # not a multiple of the 64-row tile; several CTAs
+        ip, ix = _random_pattern(n, 14, 11, hub=900 if mode == "hubs" else None)     # row 7 of "hubs" spans 29 segments
+        g = _graph(ip, ix)
     gen = torch.Generator().manual_seed(3)
     shape = (n, 128) if strands == 1 else (n, 2, 128)
     x = torch.randn(*shape, generator=gen)
@@ -452,10 +547,228 @@ def test_fused_layer_fwd_matches_fp64(strands, mode):
         assert 0.6 < float((mask > 0).double().mean()) < 0.8
         xo_ref = xo_ref * mask
     assert ogcn.max_rel(sx.cpu(), sx_ref) <= 2e-6
-    assert ogcn.max_rel(z.cpu(), z_ref) <= 1e-5 and _elementwise_rel(z, z_ref, 0.05) <= 1e-4
+    report = {"z": _panel_errors(z.cpu(), z_ref)}
     assert ogcn.max_rel(gate.cpu().reshape(g_ref.shape), g_ref) <= 1e-5
-    assert ogcn.max_rel(xo.cpu(), xo_ref) <= 1e-5 and _elementwise_rel(xo, xo_ref, 0.05) <= 1e-4
+    report["x_out"] = _panel_errors(xo.cpu(), xo_ref)
+    grid, rows = _fused_grid(n, strands, _sms())
+    stats_err = ""
     if mode == "stats":
+        assert stats.shape[0] == grid
         r = torch.relu(xo_ref).reshape(n, strands, 128)
         got = stats.double().sum(0).cpu().reshape(2, strands, 128)
-        assert ogcn.max_rel(got[0], r.sum(0)) <= 1e-5 and ogcn.max_rel(got[1], (r * r).sum(0)) <= 1e-5
+        e = (ogcn.max_rel(got[0], r.sum(0)), ogcn.max_rel(got[1], (r * r).sum(0)))
+        assert max(e) <= 1e-5
+        stats_err = " | stats max_rel %.2e %.2e" % e
+    print("fwd S=%d %s %s: %d CTAs, %d rows / CTA, %d tiles / CTA | %s%s"
+          % (strands, size, mode, grid, rows, _cdiv(rows, 64 // strands),
+             " | ".join("%s max_rel %.2e elementwise %.2e" % (k, *v) for k, v in report.items()), stats_err))
+
+
+# The backward twin (cgcn_gcn_layer_bwd).  Its panels are the forward's error structure (a CSR gather of fp32 values, then
+# a 3xTF32 128-term contraction) and get the forward test's bounds.  A column partial is a sum of signed terms over the
+# rows of a CTA: it is held to 1e-5 of the no-cancellation magnitude sum_rows |term| of its own CTA and, summed over the
+# CTAs in fp64, of the whole column.  A plain max-norm would be loose or fail on cancelling columns such as d b_g; this
+# bound catches one dropped row slot or CTA.
+_SEED, _STEP, _SITE = 1234567, 9, 0
+_NAN_BITS = 0x7FC00000                          # torch.full(..., nan)
+
+
+def _panel_errors(got, ref):
+    """The bounds of the forward's z and x_out: max-norm relative <= 1e-5, element-wise <= 1e-4."""
+    mr, er = ogcn.max_rel(got, ref), _elementwise_rel(got, ref, 0.05)
+    assert mr <= 1e-5 and er <= 1e-4, (mr, er)
+    return mr, er
+
+
+def _guarded(shape):
+    """A NaN-filled buffer with two guard rows on each side of `shape`: `(buffer, output view)`."""
+    buf = torch.full((shape[0] + 4, *shape[1:]), float("nan"), device=_dev())
+    return buf, buf[2:2 + shape[0]]
+
+
+def _guards_intact(buf, rows):
+    """The buffer's rows outside [2, 2 + rows) still hold their NaN, bit for bit."""
+    outside = torch.cat([buf[:2].reshape(-1), buf[2 + rows:].reshape(-1)])
+    return bool((outside.view(torch.int32) == _NAN_BITS).all())
+
+
+def _bits_equal(a, b):
+    return torch.equal(a.view(torch.int32), b.view(torch.int32))
+
+
+@functools.lru_cache(maxsize=4)
+def _bwd_inputs(strands, size):
+    """Edge-case graph and fp32 inputs of one (strands, size), shared by the backward cases."""
+    n = _layer_n(strands, size)
+    _, _, g = _edge_case_graph(n, strands)
+    gen = torch.Generator().manual_seed(17 + strands)
+    shape = (n, 128) if strands == 1 else (n, 2, 128)
+    inp = {k: torch.randn(*shape, generator=gen) for k in ("dys", "dxd", "y_prev", "x_prev")}
+    inp["w"] = torch.randn(128, 128, generator=gen) * 0.12
+    inp["wg"] = torch.randn(128, generator=gen) * 0.3
+    inp["bg"] = torch.randn(1, generator=gen) * 0.1
+    return n, g, inp
+
+
+def _layer_above(g, inp, x):
+    """`<G, (A_hat x) W> + <dxd, x>` with G = D dys: its gradient in x, A_hat^T G W^T + dxd, is what the kernel computes as
+    (P dys) W^T + dxd.  A_hat = D^-1 P is written out per strand from the graph's CSR on the window index, so the
+    reference does not rely on the pattern being symmetric; the kernel does."""
+    rp, ci = g.csr_numpy()
+    n, s = x.shape[0], x.shape[1]
+    deg = torch.from_numpy(np.diff(rp)).double()
+    rows = torch.repeat_interleave(torch.arange(n), deg.long())
+    a_hat = torch.sparse_coo_tensor(torch.stack([rows, torch.from_numpy(ci).long()]), 1.0 / deg[rows], (n, n)).coalesce()
+    ax = torch.sparse.mm(a_hat, x.reshape(n, s * 128)).reshape(n, s, 128)
+    G = deg[:, None, None] * inp["dys"].double().reshape(n, s, 128)
+    return (G * (ax @ inp["w"].double())).sum() + (inp["dxd"].double().reshape(n, s, 128) * x).sum()
+
+
+@functools.lru_cache(maxsize=3)
+def _bwd_mid_reference(strands, size, gate_off, p):
+    """fp64 autograd of the layer below (tanh, gate, blend, dropout with the kernel's own keep-mask) under the layer
+    above, from the fp32 values handed to the kernel.  Returns the kernel's z_prev = fp32(z) and g_prev = fp32(g), and
+    the expected dy = y_prev.grad, dxd_out = x_prev.grad, dgp = d loss / d(z . wg + bg) and z."""
+    from chromegcn_b200 import ops
+    n, g, inp = _bwd_inputs(strands, size)
+    y_prev = inp["y_prev"].double().reshape(n, strands, 128).requires_grad_(True)
+    x_prev = inp["x_prev"].double().reshape(n, strands, 128).requires_grad_(True)
+    wg = inp["wg"].double().requires_grad_(True)
+    bg = inp["bg"].double().requires_grad_(True)
+    z = torch.tanh(y_prev)
+    a = z @ wg + bg
+    a.retain_grad()
+    gate = torch.ones_like(a) if gate_off else torch.sigmoid(a)
+    x_l = (1 - gate)[..., None] * x_prev + gate[..., None] * z
+    if p > 0:
+        mask = ops.dropout_mask(n, strands, 128, p, _SEED, _STEP, _SITE, _dev()).cpu().double()
+        assert 0.6 < float((mask > 0).double().mean()) < 0.8
+        x_l = x_l * mask
+    _layer_above(g, inp, x_l).backward()
+    if gate_off:
+        assert a.grad is None and wg.grad is None and bg.grad is None
+    dgp = torch.zeros(n, strands, dtype=torch.float64) if gate_off else a.grad
+    return {"z_prev": z.detach().float(), "g_prev": gate.detach().float(), "dy": y_prev.grad, "dxd": x_prev.grad,
+            "dgp": dgp, "z": z.detach()}
+
+
+def _run_bwd_mid(strands, size, gate_off, p, dxd_out):
+    """cgcn_gcn_layer_bwd with the layer below, every output inside NaN guard rows (the partials inside a buffer of one
+    row per SM, more than the kernel has CTAs).  `dxd_out`: "new" (a panel of its own), "in_place" (the dxd panel
+    itself, as the model runs it) or None.  Returns host copies of (dys_out, dxd_out, partial)."""
+    from chromegcn_b200 import ops
+    n, g, inp = _bwd_inputs(strands, size)
+    ref = _bwd_mid_reference(strands, size, gate_off, p)
+    d = {k: v.to(_dev()) for k, v in inp.items()}
+    shape = d["dys"].shape
+    dys_buf, dys_out = _guarded(shape)
+    part_buf, part_out = _guarded((_sms(), 2 * 128 + 4))
+    dxd, dxd_buf, dxd_o = d["dxd"], None, None
+    if dxd_out == "new":
+        dxd_buf, dxd_o = _guarded(shape)
+    elif dxd_out == "in_place":
+        dxd_buf, dxd = _guarded(shape)
+        dxd.copy_(d["dxd"])
+        dxd_o = dxd
+    got = ops.gcn_layer_bwd(g, d["dys"], dxd, d["w"], ref["z_prev"].reshape(shape).to(_dev()), d["x_prev"],
+                            ref["g_prev"].to(_dev()), d["wg"], gate_off, p, _SEED, _STEP, _SITE,
+                            dys_out=dys_out, dxd_out=dxd_o, partial=part_out)
+    assert got[0] is dys_out and got[1] is dxd_o
+    parts = got[2].shape[0]
+    torch.cuda.synchronize()
+    assert _guards_intact(dys_buf, n) and _guards_intact(part_buf, parts)
+    assert dxd_buf is None or _guards_intact(dxd_buf, n)
+    return dys_out.cpu(), (None if dxd_o is None else dxd_o.cpu()), got[2].cpu()
+
+
+@pytest.mark.parametrize("mode", ["plain", "gate_off", "dropout", "in_place", "no_dxd_out"])
+@pytest.mark.parametrize("strands", [1, 2])
+@pytest.mark.parametrize("size", ["one_tile", "multi_tile"])
+def test_fused_layer_bwd_mid_matches_fp64(size, strands, mode):
+    """cgcn_gcn_layer_bwd with the layer below (fused_layer_kernel<S, BWD_MID>: gather u = P dys, u W^T on the tensor
+    cores, + dxd, then the dropout / gate / tanh backward of the layer below and its column partials for d b, d w_g,
+    d b_g) against fp64 autograd, on the edge-case graph with one and with several tiles per CTA.  The kernel must write
+    nothing outside its outputs, repeat itself bit for bit (CSR-order gathers, fixed-order partials), and give the same
+    bits when dxd_out is the dxd panel itself or absent."""
+    gate_off, p = mode == "gate_off", (0.3 if mode == "dropout" else 0.0)
+    dxd_mode = {"in_place": "in_place", "no_dxd_out": None}.get(mode, "new")
+    n, g, _ = _bwd_inputs(strands, size)
+    ref = _bwd_mid_reference(strands, size, gate_off, p)
+    grid, rows = _fused_grid(n, strands, _sms())
+    dys, dxd, part = _run_bwd_mid(strands, size, gate_off, p, dxd_mode)
+    again = _run_bwd_mid(strands, size, gate_off, p, dxd_mode)
+    assert _bits_equal(dys, again[0]) and _bits_equal(part, again[2]) and (dxd is None or _bits_equal(dxd, again[1]))
+    if dxd_mode != "new":
+        plain = _run_bwd_mid(strands, size, gate_off, p, "new")
+        assert _bits_equal(dys, plain[0]) and _bits_equal(part, plain[2]) and (dxd is None or _bits_equal(dxd, plain[1]))
+    assert part.shape[0] == grid
+    # dys_out = D^-1 dy, compared as D dys_out against dy: rows with few entries (large 1/D) would otherwise set the
+    # max-norm and the element-wise floor for all the others
+    deg = torch.from_numpy(np.diff(g.csr_numpy()[0])).double()
+    report = {"dys_out": _panel_errors(dys.double().reshape(n, strands, 128) * deg[:, None, None], ref["dy"])}
+    if dxd is not None:
+        if gate_off:
+            assert bool((dxd == 0).all())
+        else:
+            report["dxd_out"] = _panel_errors(dxd.reshape(n, strands, 128), ref["dxd"])
+    # partial columns d b | d w_g | d b_g, then 3 zeros; per CTA (its window rows, both strands) and in total
+    dgp = ref["dgp"]
+    terms = torch.cat([ref["dy"], dgp[..., None] * ref["z"], dgp[..., None]], -1)
+    cta = torch.arange(n) // rows
+    want = torch.zeros(grid, 257, dtype=torch.float64).index_add_(0, cta, terms.sum(1))
+    bound = 1e-5 * torch.zeros(grid, 257, dtype=torch.float64).index_add_(0, cta, terms.abs().sum(1))
+    got = part.double()
+    assert bool((got[:, 257:] == 0).all())
+    if gate_off:
+        assert bool((got[:, 128:257] == 0).all())
+    worst = []
+    for diff, bnd in (((got[:, :257] - want).abs(), bound), ((got[:, :257].sum(0) - want.sum(0)).abs(), bound.sum(0))):
+        assert bool((diff <= bnd).all()), (diff - bnd).max()
+        worst.append(float((diff / bnd)[bnd > 0].max()))
+    print("bwd_mid S=%d %s %s: parts %d, %d rows / CTA, %d tiles / CTA | %s | partials err/bound: per CTA %.3f, total %.3f"
+          % (strands, size, mode, grid, rows, _cdiv(rows, 64 // strands),
+             " | ".join("%s max_rel %.2e elementwise %.2e" % (k, *v) for k, v in report.items()), *worst))
+
+
+@pytest.mark.parametrize("strands", [1, 2])
+@pytest.mark.parametrize("size", ["one_tile", "multi_tile"])
+def test_fused_layer_bwd_input_matches_fp64(size, strands):
+    """cgcn_gcn_layer_bwd without the layer below (fused_layer_kernel<S, BWD_INPUT>): dx_out = (P dys) W^T + dxd is
+    d loss / d x of the layer above, against fp64 autograd; nothing written outside dx_out, bit-identical when repeated."""
+    from chromegcn_b200 import ops
+    n, g, inp = _bwd_inputs(strands, size)
+    x = torch.zeros(n, strands, 128, dtype=torch.float64, requires_grad=True)
+    _layer_above(g, inp, x).backward()
+    d = {k: v.to(_dev()) for k, v in inp.items()}
+    outs = []
+    for _ in range(2):
+        buf, dx = _guarded(d["dys"].shape)
+        assert ops.gcn_layer_bwd(g, d["dys"], d["dxd"], d["w"], dx_out=dx) is dx
+        torch.cuda.synchronize()
+        assert _guards_intact(buf, n)
+        outs.append(dx.cpu())
+    assert _bits_equal(outs[0], outs[1])
+    grid, rows = _fused_grid(n, strands, _sms())
+    print("bwd_input S=%d %s: %d CTAs, %d rows / CTA, %d tiles / CTA | dx_out max_rel %.2e elementwise %.2e"
+          % (strands, size, grid, rows, _cdiv(rows, 64 // strands), *_panel_errors(outs[0].reshape(n, strands, 128), x.grad)))
+
+
+def test_fused_layer_bwd_rejects_invalid_arguments():
+    """cgcn_gcn_layer_bwd refuses, before it launches anything, a dys_out that aliases the gathered panel, a missing
+    layer-below tensor, a weighted graph and a dropout probability outside [0, 1) -- NaN included, which would otherwise
+    switch dropout off without a word."""
+    from chromegcn_b200 import _lib, ops
+    from chromegcn_b200.graph import HiCGraph
+    n, g, inp = _bwd_inputs(2, "one_tile")
+    ref = _bwd_mid_reference(2, "one_tile", False, 0.0)
+    d = {k: v.to(_dev()) for k, v in inp.items()}
+    below = dict(z_prev=ref["z_prev"].to(_dev()), x_prev=d["x_prev"], g_prev=ref["g_prev"].to(_dev()), wg_prev=d["wg"])
+    bad = [dict(below, dys_out=d["dys"])] + [dict(below, **{k: None}) for k in ("x_prev", "g_prev", "wg_prev")]
+    bad += [dict(below, dropout_p=p) for p in (-0.1, 1.0, 1.5, float("nan"))]
+    weighted = HiCGraph(g.rowptr, g.colidx, n, g.nnz, vals=torch.ones(g.nnz, device=_dev()),
+                        row_inv=torch.ones(n, device=_dev()))
+    before = _lib.launch_count()
+    for graph, kw in [(g, k) for k in bad] + [(weighted, below), (weighted, {})]:
+        with pytest.raises(_lib.ChromeGCNNativeError):
+            ops.gcn_layer_bwd(graph, d["dys"], d["dxd"], d["w"], **kw)
+    assert _lib.launch_count() == before

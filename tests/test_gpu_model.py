@@ -242,39 +242,59 @@ def test_dropout_training_matches_oracle_with_injected_masks():
 
 
 def test_large_graph_against_oracle():
-    """A config-1 sized chromosome (N = 20 000, 520 k stored entries): fused step vs the CPU oracle in fp64."""
+    """Config-1 sized chromosomes (N = 20 000) vs the CPU oracle in fp64, through both entry points: the fused step (both
+    strands in one cgcn_train_step) and the module API (finetune.py:41-48: one strand per call, BCE on the mean,
+    backward).  With 500 k Hi-C edges (520 k stored entries, mean degree 26) every layer runs as three kernels.  With
+    400 k (mean degree 21) every layer runs as the fused layer kernel, and on 148 SMs each CTA of it runs several tiles:
+    136 rows = 3 tiles of 64 with one strand, 5 of 32 with two, the last tile holding 8 rows."""
     from chromegcn_b200 import synthetic
     from chromegcn_b200.chrome_models import ChromeGCN
     from chromegcn_b200.engine import ChromosomeEngine
     from chromegcn_b200.graph import HiCGraph
     from oracle import adjacency as oadj
-    h = synthetic.make_hic("chr22")
-    ip, ix = oadj.build_adjacency_numpy(h.window_starts, h.bin1, h.bin2, h.val, h.norm, 1, 500000)
-    n = ip.shape[0] - 1
-    feats = synthetic.make_features("chr22", n)
-    torch.manual_seed(0)
-    om = ogcn.ChromeGCNOracle(128, 128, synthetic.NCLASS, 0.0, True, 2)
-    ogcn.stress_init_(om)
-    m = ChromeGCN(128, 128, synthetic.NCLASS, 0.0, True, 2)
-    m.load_state_dict(om.state_dict())
-    m = m.to(_dev()).train()
-    om = om.double().train()
-    adj = ogcn.coo_adjacency(ip, ix, torch.float64)
-    lo, prob_o, pred_o, _ = ogcn.chromosome_step(om, feats["forward"].double(), feats["backward"].double(),
-                                                 feats["target"].double(), adj, None, True)
-    g = HiCGraph.from_csr_pattern(ip, ix, _dev())
-    assert g.nnz == ip[-1] + n
-    eng = ChromosomeEngine(m, 2)
-    probs = torch.empty(n, synthetic.NCLASS, device=_dev())
-    loss = torch.zeros(1, device=_dev())
-    out, _ = eng.run(g, eng.pack(feats["forward"].to(_dev()), feats["backward"].to(_dev())), feats["target"].to(_dev()),
-                     probs, loss, train=True)
-    assert ogcn.max_rel(out.mean(1).cpu(), pred_o) <= FWD_TOL
-    assert ogcn.max_rel(probs.cpu(), prob_o) <= FWD_TOL
-    assert abs(loss.item() - lo) <= FWD_TOL * abs(lo)
-    for (k, p), (_, q) in zip(m.named_parameters(), om.named_parameters()):
-        err = ogcn.max_rel(p.grad.cpu(), q.grad)
-        assert err <= 5e-5, (k, err)
+    for hic_edges, fused in ((500000, False), (400000, True)):
+        h = synthetic.make_hic("chr22", hic_edges=hic_edges)
+        ip, ix = oadj.build_adjacency_numpy(h.window_starts, h.bin1, h.bin2, h.val, h.norm, 1, hic_edges)
+        n = ip.shape[0] - 1
+        feats = synthetic.make_features("chr22", n)
+        torch.manual_seed(0)
+        om = ogcn.ChromeGCNOracle(128, 128, synthetic.NCLASS, 0.0, True, 2)
+        ogcn.stress_init_(om)
+        sd = {k: v.clone() for k, v in om.state_dict().items()}
+        m = ChromeGCN(128, 128, synthetic.NCLASS, 0.0, True, 2)
+        m.load_state_dict(sd)
+        m = m.to(_dev()).train()
+        om = om.double().train()
+        adj = ogcn.coo_adjacency(ip, ix, torch.float64)
+        lo, prob_o, pred_o, _ = ogcn.chromosome_step(om, feats["forward"].double(), feats["backward"].double(),
+                                                     feats["target"].double(), adj, None, True)
+        g = HiCGraph.from_csr_pattern(ip, ix, _dev())
+        assert g.nnz == ip[-1] + n
+        assert (g.nnz <= 24 * n) == fused          # FUSED_MAX_DEGREE (csrc/model.cu) selects the layer path
+        eng = ChromosomeEngine(m, 2)
+        probs = torch.empty(n, synthetic.NCLASS, device=_dev())
+        loss = torch.zeros(1, device=_dev())
+        out, _ = eng.run(g, eng.pack(feats["forward"].to(_dev()), feats["backward"].to(_dev())), feats["target"].to(_dev()),
+                         probs, loss, train=True)
+        # the module API on the same model and inputs
+        m1 = ChromeGCN(128, 128, synthetic.NCLASS, 0.0, True, 2)
+        m1.load_state_dict(sd)
+        m1 = m1.to(_dev()).train()
+        _, pf, _, _ = m1(feats["forward"].to(_dev()), g, None)
+        _, pr, _, _ = m1(feats["backward"].to(_dev()), g, None)
+        pred1 = (pf + pr) / 2
+        loss1 = F.binary_cross_entropy_with_logits(pred1, feats["target"].to(_dev()))
+        loss1.backward()
+        for arm, model, pred, prob, l in (("engine", m, out.mean(1), probs, loss.item()),
+                                          ("module", m1, pred1.detach(), torch.sigmoid(pred1.detach()), loss1.item())):
+            errs = [ogcn.max_rel(pred.cpu(), pred_o), ogcn.max_rel(prob.cpu(), prob_o), abs(l - lo) / abs(lo)]
+            assert max(errs) <= FWD_TOL, (hic_edges, arm, errs)
+            for (k, p), (_, q) in zip(model.named_parameters(), om.named_parameters()):
+                err = ogcn.max_rel(p.grad.cpu(), q.grad)
+                assert err <= 5e-5, (hic_edges, arm, k, err)
+                errs.append(err)
+            print("large graph, %d Hi-C edges, %s: pred %.2e prob %.2e loss %.2e, worst gradient %.2e"
+                  % (hic_edges, arm, *errs[:3], max(errs[3:])))
 
 
 def _auc_aupr(targets, preds):
