@@ -94,6 +94,18 @@ struct TcImageSpec {
 };
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// Peer gather (one graph row-partitioned over the GPUs of an NVLink box): the gathered panel lives in the ranks'
+// exchange buffers (cgcn_peer_panel); rank r owns global rows [begin[r], begin[r+1]) at base[r].  Passed by value in
+// kernel parameters, read with peer_row().
+struct PeerTable {
+  int world;
+  int begin[CGCN_MAX_PEERS + 1];
+  const float* base[CGCN_MAX_PEERS];
+};
+
+// Fills *t from pp and checks it against this rank's graph of n_local rows; error messages start with `who`.
+int peer_table(PeerTable* t, const cgcn_peer_panel* pp, int n_local, const char* who);
+
 // bump allocator over a caller-provided workspace
 struct Arena {
   char* base;
@@ -133,6 +145,16 @@ __device__ __forceinline__ float inv_degree(const int32_t* __restrict__ rowptr, 
 // 1/deg from the pattern, or the stored 1/rowsum of a weighted graph
 __device__ __forceinline__ float row_scale(const int32_t* __restrict__ rowptr, const float* __restrict__ row_inv, int row) {
   return row_inv != nullptr ? __ldg(row_inv + row) : inv_degree(rowptr, row);
+}
+
+// Row c of a panel of pitch_floats floats per row, spread over the ranks of t: the owner is counted with
+// CGCN_MAX_PEERS - 1 compares.  A kernel that takes the table as a parameter of its own declares it __grid_constant__;
+// dynamically indexed, a by-value parameter of this size is otherwise copied to local memory.
+__device__ __forceinline__ const float* peer_row(const PeerTable& t, int c, size_t pitch_floats) {
+  int o = 0;
+#pragma unroll
+  for (int r = 1; r < CGCN_MAX_PEERS; ++r) o += (r < t.world && c >= t.begin[r]) ? 1 : 0;
+  return t.base[o] + static_cast<size_t>(c - t.begin[o]) * pitch_floats;
 }
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }

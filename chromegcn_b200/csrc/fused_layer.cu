@@ -265,10 +265,7 @@ __global__ void __launch_bounds__(THREADS, 1) fused_layer_kernel(const Args a) {
         const int c = __shfl_sync(0xffffffffu, cols, min(k0 + u, last));
         const float* p;
         if constexpr (PEER) {                      // owner of global row c: NVLink load from its exchange buffer
-          int o = 0;
-#pragma unroll
-          for (int r = 1; r < CGCN_MAX_PEERS; ++r) o += (r < a.peer_world && c >= a.peer_begin[r]) ? 1 : 0;
-          p = a.peer_base[o] + static_cast<size_t>(c - a.peer_begin[o]) * (S * 128) + lane * 4;
+          p = peer_row(a.peer, c, S * 128) + lane * 4;
         } else {
           p = gbase + static_cast<size_t>(c) * (S * 128);
         }
@@ -606,32 +603,17 @@ static int launch_mode(const fl::Args& a, int mode, int grid, cudaStream_t strea
 }
 
 int fused_layer_launch(fl::Args a, int S, int mode, int* grid_out, cudaStream_t stream) {
-  CGCN_REQUIRE(a.rowptr && a.colidx && (a.gsrc || a.peer_world > 0) && a.w, "fused layer: null graph / panel / weight");
+  CGCN_REQUIRE(a.rowptr && a.colidx && (a.gsrc || a.peer.world > 0) && a.w, "fused layer: null graph / panel / weight");
   CGCN_REQUIRE(S == 1 || S == 2, "fused layer: strands=%d", S);
   int rows = 0;
   const int grid = fused_layer_grid(a.n, S, &rows);
   a.rows_per_cta = rows;
   if (grid_out) *grid_out = grid;
   if (a.n <= 0) return CGCN_OK;
-  const bool peer = a.peer_world > 0;
-  if (peer) a.gsrc = a.peer_base[0];
+  const bool peer = a.peer.world > 0;
+  if (peer) a.gsrc = a.peer.base[0];
   if (S == 1) return peer ? launch_mode<1, true>(a, mode, grid, stream) : launch_mode<1, false>(a, mode, grid, stream);
   return peer ? launch_mode<2, true>(a, mode, grid, stream) : launch_mode<2, false>(a, mode, grid, stream);
-}
-
-int fused_layer_set_peer(fl::Args* a, const cgcn_peer_panel* pp, int n_local) {
-  CGCN_REQUIRE(pp != nullptr && pp->world >= 1 && pp->world <= CGCN_MAX_PEERS && pp->rank >= 0 && pp->rank < pp->world,
-               "fused layer: bad peer panel");
-  a->peer_world = pp->world;
-  for (int r = 0; r < pp->world; ++r) {
-    CGCN_REQUIRE(pp->base[r] != nullptr && pp->row_begin[r] <= pp->row_begin[r + 1], "fused layer: bad peer block %d", r);
-    a->peer_base[r] = pp->base[r];
-    a->peer_begin[r] = pp->row_begin[r];
-  }
-  a->peer_begin[pp->world] = pp->row_begin[pp->world];
-  CGCN_REQUIRE(pp->row_begin[pp->rank + 1] - pp->row_begin[pp->rank] == n_local, "fused layer: graph has %d rows, peer block %d",
-               n_local, pp->row_begin[pp->rank + 1] - pp->row_begin[pp->rank]);
-  return CGCN_OK;
 }
 
 }  // namespace cgcn

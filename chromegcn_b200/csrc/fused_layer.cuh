@@ -35,19 +35,16 @@ struct Args {
   float* dys_out;              // D^-1 dy_{l-1}
   float* dxd_out;              // (1-g_{l-1}) dh_{l-1} or NULL (may alias dxd_in)
   float* dx_out;               // BWD_INPUT: d loss / d x_in
-  // ---- peer gather (one graph row-partitioned over the GPUs of an NVLink box): the gathered panel lives in the ranks'
-  // exchange buffers (cgcn_peer_panel); rank r owns global rows [peer_begin[r], peer_begin[r+1]) at peer_base[r].
-  // peer_world == 0: plain gather from gsrc.
-  int peer_world;
-  int peer_begin[CGCN_MAX_PEERS + 1];
-  const float* peer_base[CGCN_MAX_PEERS];
+  PeerTable peer;              // gather from the ranks' exchange buffers; peer.world == 0: plain gather from gsrc
 };
+static_assert(sizeof(Args) == 328 && offsetof(Args, peer) == 224 && offsetof(Args, peer.begin) == 228 &&
+                  offsetof(Args, peer.base) == 264,
+              "fused layer argument block layout");
 
 }  // namespace fl
 
 bool fused_layer_supported(int d, const cgcn_graph* g);
 int fused_layer_grid(int n, int S, int* rows_per_cta_out);
 int fused_layer_launch(fl::Args a, int S, int mode, int* grid_out, cudaStream_t stream);
-int fused_layer_set_peer(fl::Args* a, const cgcn_peer_panel* pp, int n_local);
 
 }  // namespace cgcn

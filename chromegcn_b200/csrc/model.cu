@@ -406,7 +406,7 @@ static int fwd_layer(const Ctx& c, int l, const float* gather_src) {
     a.colidx = m->graph.colidx;
     a.n = c.n;
     a.gsrc = gather_src;
-    if (c.dist && m->peer != nullptr) CGCN_TRY(fused_layer_set_peer(&a, m->peer, c.n));      // neighbour rows over NVLink
+    if (c.dist && m->peer != nullptr) CGCN_TRY(peer_table(&a.peer, m->peer, c.n, "fused layer"));  // neighbour rows over NVLink
     a.w = m->params.gc_w[l];
     a.w_transposed = 0;
     a.xin = xin;
@@ -577,7 +577,7 @@ static int bwd_propagate(const Ctx& c, int l_from, const float* gather, int* par
   a.colidx = m->graph.colidx;
   a.n = c.n;
   a.gsrc = gather;
-  if (c.dist && m->peer != nullptr) CGCN_TRY(fused_layer_set_peer(&a, m->peer, c.n));
+  if (c.dist && m->peer != nullptr) CGCN_TRY(peer_table(&a.peer, m->peer, c.n, "fused layer"));
   a.w = m->params.gc_w[l_from];
   a.w_transposed = 1;
   a.dxd_in = ws + lay.dC;

@@ -23,15 +23,42 @@ namespace cgcn {
 constexpr int SPMM_WARPS = 8;
 constexpr int LONG_ROW = 512;
 
-template <int VEC, bool WEIGHTED>
+// Where the gathered rows come from: the local panel x (pattern, or weighted by vals), or the panel spread over the
+// ranks' exchange buffers (PeerTable).
+constexpr int ROWS_PATTERN = 0, ROWS_WEIGHTED = 1, ROWS_PEER = 2;
+
+__device__ __forceinline__ const float* shfl_ptr(const float* p, int src) {
+  const unsigned long long v = reinterpret_cast<unsigned long long>(p);
+  const unsigned lo = __shfl_sync(0xffffffffu, static_cast<unsigned>(v), src);
+  const unsigned hi = __shfl_sync(0xffffffffu, static_cast<unsigned>(v >> 32), src);
+  return reinterpret_cast<const float*>((static_cast<unsigned long long>(hi) << 32) | lo);
+}
+
+// acc += the rows of entries [begin, end), in CSR order.  The local sources broadcast the column index and form the
+// address after the shuffle; the peer source resolves the owner of its lane's column once per 32 entries and
+// broadcasts the 64-bit row pointer, which keeps the lookup off the per-neighbour path.
+template <int VEC, int SRC>
 __device__ __forceinline__ void gather_range(const int32_t* __restrict__ colidx, const float* __restrict__ vals,
-                                             const float* __restrict__ x, int begin, int end, int lane, float4 (&acc)[VEC]) {
+                                             const float* __restrict__ x, const PeerTable& peer, int begin, int end,
+                                             int lane, float4 (&acc)[VEC]) {
+  constexpr bool WEIGHTED = SRC == ROWS_WEIGHTED;
   constexpr int UNROLL = (VEC >= 8) ? 1 : (8 / VEC);
   constexpr size_t PITCH = static_cast<size_t>(VEC) * 128;
   for (int base = begin; base < end; base += 32) {
     const int mine = (base + lane < end) ? __ldg(colidx + base + lane) : 0;
     float wmine = 1.0f;
     if (WEIGHTED) wmine = (base + lane < end) ? __ldg(vals + base + lane) : 0.0f;
+    const float* pmine = nullptr;
+    if (SRC == ROWS_PEER) pmine = peer_row(peer, mine, PITCH);   // lanes past the end: never broadcast
+    auto row = [&](int k, float& w) -> const float* {       // this lane's part of the batch's k-th row, and its weight
+      if (SRC == ROWS_PEER) {
+        w = 1.0f;
+        return shfl_ptr(pmine, k) + lane * 4;
+      }
+      const int c = __shfl_sync(0xffffffffu, mine, k);
+      w = WEIGHTED ? __shfl_sync(0xffffffffu, wmine, k) : 1.0f;
+      return x + static_cast<size_t>(c) * PITCH + lane * 4;
+    };
     const int cnt = min(32, end - base);
     int k = 0;
     for (; k + UNROLL <= cnt; k += UNROLL) {
@@ -39,9 +66,7 @@ __device__ __forceinline__ void gather_range(const int32_t* __restrict__ colidx,
       float w[UNROLL];
 #pragma unroll
       for (int u = 0; u < UNROLL; ++u) {
-        const int c = __shfl_sync(0xffffffffu, mine, k + u);
-        w[u] = WEIGHTED ? __shfl_sync(0xffffffffu, wmine, k + u) : 1.0f;
-        const float* p = x + static_cast<size_t>(c) * PITCH + lane * 4;
+        const float* p = row(k + u, w[u]);
 #pragma unroll
         for (int q = 0; q < VEC; ++q) v[u][q] = ldg4(p + q * 128);
       }
@@ -63,10 +88,9 @@ __device__ __forceinline__ void gather_range(const int32_t* __restrict__ colidx,
         }
       }
     }
-    for (; k < cnt; ++k) {
-      const int c = __shfl_sync(0xffffffffu, mine, k);
-      const float w1 = WEIGHTED ? __shfl_sync(0xffffffffu, wmine, k) : 1.0f;
-      const float* p = x + static_cast<size_t>(c) * PITCH + lane * 4;
+    for (; k < cnt; ++k) {                         // fmaf(1, v, acc) == acc + v: one tail for every source
+      float w1;
+      const float* p = row(k, w1);
 #pragma unroll
       for (int q = 0; q < VEC; ++q) {
         const float4 v = ldg4(p + q * 128);
@@ -79,19 +103,35 @@ __device__ __forceinline__ void gather_range(const int32_t* __restrict__ colidx,
   }
 }
 
-template <int VEC, bool WEIGHTED>
+// x (local sources) or peer (ROWS_PEER) is the gathered panel; vals / row_inv are read by ROWS_WEIGHTED only.
+template <int VEC, int SRC>
 __global__ void __launch_bounds__(SPMM_WARPS * 32, (VEC <= 2) ? 5 : 2)
 spmm_pattern_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ colidx, int n,
                     const float* __restrict__ x, float* __restrict__ out, int scale_mode,
                     const float* __restrict__ residual, const float* __restrict__ vals,
-                    const float* __restrict__ row_inv) {
+                    const float* __restrict__ row_inv, const __grid_constant__ PeerTable peer) {
   pdl_grid_sync();
+  constexpr bool WEIGHTED = SRC == ROWS_WEIGHTED;
   constexpr size_t PITCH = static_cast<size_t>(VEC) * 128;
   __shared__ float4 red[SPMM_WARPS][VEC][32];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   const int row0 = blockIdx.x * SPMM_WARPS;
   const int row = row0 + warp;
+  auto scale = [&](int r, int d) {
+    return (scale_mode != 1) ? 1.0f : (WEIGHTED ? __ldg(row_inv + r) : (d > 0 ? __fdiv_rn(1.0f, static_cast<float>(d)) : 1.0f));
+  };
+  auto finish = [&](int r, int q, float s, float4 t) {          // out[r] = s * sum (+ residual[r]), float4 q of the lane
+    t = make_float4(t.x * s, t.y * s, t.z * s, t.w * s);
+    if (residual != nullptr) {
+      const float4 e = ldg4(residual + static_cast<size_t>(r) * PITCH + lane * 4 + q * 128);
+      t.x += e.x;
+      t.y += e.y;
+      t.z += e.z;
+      t.w += e.w;
+    }
+    st4(out + static_cast<size_t>(r) * PITCH + lane * 4 + q * 128, t);
+  };
 
   int start = 0, end = 0;
   if (row < n) {
@@ -103,22 +143,10 @@ spmm_pattern_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restric
     float4 acc[VEC];
 #pragma unroll
     for (int q = 0; q < VEC; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-    gather_range<VEC, WEIGHTED>(colidx, vals, x, start, end, lane, acc);
-    const float s = (scale_mode != 1) ? 1.0f
-                    : (WEIGHTED ? __ldg(row_inv + row) : (deg > 0 ? __fdiv_rn(1.0f, static_cast<float>(deg)) : 1.0f));
-    float* o = out + static_cast<size_t>(row) * PITCH + lane * 4;
+    gather_range<VEC, SRC>(colidx, vals, x, peer, start, end, lane, acc);
+    const float s = scale(row, deg);
 #pragma unroll
-    for (int q = 0; q < VEC; ++q) {
-      float4 r = make_float4(acc[q].x * s, acc[q].y * s, acc[q].z * s, acc[q].w * s);
-      if (residual != nullptr) {
-        const float4 e = ldg4(residual + static_cast<size_t>(row) * PITCH + lane * 4 + q * 128);
-        r.x += e.x;
-        r.y += e.y;
-        r.z += e.z;
-        r.w += e.w;
-      }
-      st4(o + q * 128, r);
-    }
+    for (int q = 0; q < VEC; ++q) finish(row, q, s, acc[q]);
   }
 
   // hub rows: any row of this CTA longer than LONG_ROW is shared by all 8 warps
@@ -135,12 +163,12 @@ spmm_pattern_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restric
     float4 acc[VEC];
 #pragma unroll
     for (int q = 0; q < VEC; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-    gather_range<VEC, WEIGHTED>(colidx, vals, x, b, e, lane, acc);
+    gather_range<VEC, SRC>(colidx, vals, x, peer, b, e, lane, acc);
 #pragma unroll
     for (int q = 0; q < VEC; ++q) red[warp][q][lane] = acc[q];
     __syncthreads();
     if (warp == 0) {
-      const float s = (scale_mode != 1) ? 1.0f : (WEIGHTED ? __ldg(row_inv + lrow) : __fdiv_rn(1.0f, static_cast<float>(ldeg)));
+      const float s = scale(lrow, ldeg);
 #pragma unroll
       for (int q = 0; q < VEC; ++q) {
         float4 t = red[0][q][lane];
@@ -151,202 +179,72 @@ spmm_pattern_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restric
           t.z += u.z;
           t.w += u.w;
         }
-        t = make_float4(t.x * s, t.y * s, t.z * s, t.w * s);
-        if (residual != nullptr) {
-          const float4 e4 = ldg4(residual + static_cast<size_t>(lrow) * PITCH + lane * 4 + q * 128);
-          t.x += e4.x;
-          t.y += e4.y;
-          t.z += e4.z;
-          t.w += e4.w;
-        }
-        st4(out + static_cast<size_t>(lrow) * PITCH + lane * 4 + q * 128, t);
+        finish(lrow, q, s, t);
       }
     }
     __syncthreads();
   }
 }
 
-
-// ------------------------------------------------------------------------------------------------
-// Peer-memory variant: the gathered panel is spread over the exchange buffers of the ranks that share one
-// row-partitioned graph (cgcn_peer_panel).  Same warp-per-row schedule; each lane resolves the owner of ITS
-// column index once (<= 7 compares against the block boundaries) into a row pointer, and the 64-bit pointer is
-// what gets broadcast by shuffle.  Rows owned by this rank come from local HBM / L2, the others arrive as NVLink
-// loads from the owner's memory -- there is no all-gathered copy of the panel.
-struct PeerTable {
-  const float* base[CGCN_MAX_PEERS];
-  int begin[CGCN_MAX_PEERS + 1];
-  int world;
-};
-
-template <int VEC>
-__device__ __forceinline__ const float* peer_row(const PeerTable& t, int c) {
-  int o = 0;
-#pragma unroll
-  for (int r = 1; r < CGCN_MAX_PEERS; ++r) o += (r < t.world && c >= t.begin[r]) ? 1 : 0;
-  return t.base[o] + static_cast<size_t>(c - t.begin[o]) * (static_cast<size_t>(VEC) * 128);
+// One launch of spmm_pattern_kernel over g->n > 0 rows, after the entry point has checked its arguments.
+// cgcn_spmm takes widths 128 x {1, 2, 3, 4, 6, 8}, cgcn_spmm_peer 128 x {1, 2, 4, 8}.
+static int spmm_run(const cgcn_graph* g, int src, const float* x, const PeerTable& peer, float* out, int width,
+                    int scale_mode, const float* residual, cudaStream_t stream) {
+  const dim3 grid((g->n + SPMM_WARPS - 1) / SPMM_WARPS), block(SPMM_WARPS * 32);
+#define SPMM_CASE(SRC, V)                                                                                          \
+  case SRC * 16 + V:                                                                                               \
+    CGCN_CUDA(launch_k(spmm_pattern_kernel<V, SRC>, grid, block, 0, stream, g->rowptr, g->colidx, g->n, x, out,    \
+                       scale_mode, residual, g->vals, g->row_inv, peer));                                          \
+    break;
+#define SPMM_LOCAL_CASES(SRC) SPMM_CASE(SRC, 1) SPMM_CASE(SRC, 2) SPMM_CASE(SRC, 3) SPMM_CASE(SRC, 4) SPMM_CASE(SRC, 6) SPMM_CASE(SRC, 8)
+  switch (src * 16 + width / 128) {
+    SPMM_LOCAL_CASES(ROWS_PATTERN)
+    SPMM_LOCAL_CASES(ROWS_WEIGHTED)
+    SPMM_CASE(ROWS_PEER, 1)
+    SPMM_CASE(ROWS_PEER, 2)
+    SPMM_CASE(ROWS_PEER, 4)
+    SPMM_CASE(ROWS_PEER, 8)
+    default:
+      if (src == ROWS_PEER)
+        set_error("cgcn_spmm_peer: unsupported width %d (128, 256, 512 or 1024)", width);
+      else
+        set_error("cgcn_spmm: unsupported width %d", width);
+      return CGCN_ERR_INVALID;
+  }
+#undef SPMM_LOCAL_CASES
+#undef SPMM_CASE
+  return check_launch("spmm_pattern_kernel");
 }
 
-__device__ __forceinline__ const float* shfl_ptr(const float* p, int src) {
-  const unsigned long long v = reinterpret_cast<unsigned long long>(p);
-  const unsigned lo = __shfl_sync(0xffffffffu, static_cast<unsigned>(v), src);
-  const unsigned hi = __shfl_sync(0xffffffffu, static_cast<unsigned>(v >> 32), src);
-  return reinterpret_cast<const float*>((static_cast<unsigned long long>(hi) << 32) | lo);
-}
-
-template <int VEC>
-__device__ __forceinline__ void gather_range_peer(const int32_t* __restrict__ colidx, const PeerTable& t, int begin, int end,
-                                                  int lane, float4 (&acc)[VEC]) {
-  constexpr int UNROLL = (VEC >= 8) ? 1 : (8 / VEC);
-  for (int base = begin; base < end; base += 32) {
-    const bool have = base + lane < end;
-    const float* mine = have ? peer_row<VEC>(t, __ldg(colidx + base + lane)) : t.base[0];
-    const int cnt = min(32, end - base);
-    int k = 0;
-    for (; k + UNROLL <= cnt; k += UNROLL) {
-      float4 v[UNROLL][VEC];
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u) {
-        const float* p = shfl_ptr(mine, k + u) + lane * 4;
-#pragma unroll
-        for (int q = 0; q < VEC; ++q) v[u][q] = ldg4(p + q * 128);
-      }
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u)
-#pragma unroll
-        for (int q = 0; q < VEC; ++q) {
-          acc[q].x += v[u][q].x;
-          acc[q].y += v[u][q].y;
-          acc[q].z += v[u][q].z;
-          acc[q].w += v[u][q].w;
-        }
-    }
-    for (; k < cnt; ++k) {
-      const float* p = shfl_ptr(mine, k) + lane * 4;
-#pragma unroll
-      for (int q = 0; q < VEC; ++q) {
-        const float4 v = ldg4(p + q * 128);
-        acc[q].x += v.x;
-        acc[q].y += v.y;
-        acc[q].z += v.z;
-        acc[q].w += v.w;
-      }
-    }
+int peer_table(PeerTable* t, const cgcn_peer_panel* pp, int n_local, const char* who) {
+  CGCN_REQUIRE(pp != nullptr, "%s: null peer panel", who);
+  CGCN_REQUIRE(pp->world >= 1 && pp->world <= CGCN_MAX_PEERS && pp->rank >= 0 && pp->rank < pp->world,
+               "%s: peer panel world=%d rank=%d", who, pp->world, pp->rank);
+  *t = PeerTable{};
+  t->world = pp->world;
+  for (int r = 0; r < pp->world; ++r) {
+    CGCN_REQUIRE(pp->base[r] != nullptr && pp->row_begin[r] <= pp->row_begin[r + 1], "%s: bad peer block %d", who, r);
+    t->base[r] = pp->base[r];
+    t->begin[r] = pp->row_begin[r];
   }
-}
-
-template <int VEC>
-__global__ void __launch_bounds__(SPMM_WARPS * 32, (VEC <= 2) ? 5 : 2)
-spmm_peer_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ colidx, int n, const PeerTable t,
-                 float* __restrict__ out, int scale_mode, const float* __restrict__ residual) {
-  pdl_grid_sync();
-  constexpr size_t PITCH = static_cast<size_t>(VEC) * 128;
-  __shared__ float4 red[SPMM_WARPS][VEC][32];
-  const int lane = threadIdx.x & 31;
-  const int warp = threadIdx.x >> 5;
-  const int row0 = blockIdx.x * SPMM_WARPS;
-  const int row = row0 + warp;
-  int start = 0, end = 0;
-  if (row < n) {
-    start = __ldg(rowptr + row);
-    end = __ldg(rowptr + row + 1);
-  }
-  const int deg = end - start;
-  auto finish = [&](float4 (&acc)[VEC], int r, int d) {
-    const float s = (scale_mode != 1) ? 1.0f : (d > 0 ? __fdiv_rn(1.0f, static_cast<float>(d)) : 1.0f);
-#pragma unroll
-    for (int q = 0; q < VEC; ++q) {
-      float4 v = make_float4(acc[q].x * s, acc[q].y * s, acc[q].z * s, acc[q].w * s);
-      if (residual != nullptr) {
-        const float4 e = ldg4(residual + static_cast<size_t>(r) * PITCH + lane * 4 + q * 128);
-        v.x += e.x;
-        v.y += e.y;
-        v.z += e.z;
-        v.w += e.w;
-      }
-      st4(out + static_cast<size_t>(r) * PITCH + lane * 4 + q * 128, v);
-    }
-  };
-  if (row < n && deg <= LONG_ROW) {
-    float4 acc[VEC];
-#pragma unroll
-    for (int q = 0; q < VEC; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-    gather_range_peer<VEC>(colidx, t, start, end, lane, acc);
-    finish(acc, row, deg);
-  }
-  const int any_long = __syncthreads_or(row < n && deg > LONG_ROW);
-  if (!any_long) return;
-  for (int r = 0; r < SPMM_WARPS; ++r) {               // hub rows: shared by the 8 warps, fixed-order combine
-    const int lrow = row0 + r;
-    if (lrow >= n) break;
-    const int ls = __ldg(rowptr + lrow), le = __ldg(rowptr + lrow + 1);
-    const int ldeg = le - ls;
-    if (ldeg <= LONG_ROW) continue;
-    const int chunk = (ldeg + SPMM_WARPS - 1) / SPMM_WARPS;
-    const int b = min(ls + warp * chunk, le), e = min(b + chunk, le);
-    float4 acc[VEC];
-#pragma unroll
-    for (int q = 0; q < VEC; ++q) acc[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-    gather_range_peer<VEC>(colidx, t, b, e, lane, acc);
-#pragma unroll
-    for (int q = 0; q < VEC; ++q) red[warp][q][lane] = acc[q];
-    __syncthreads();
-    if (warp == 0) {
-      float4 tot[VEC];
-#pragma unroll
-      for (int q = 0; q < VEC; ++q) {
-        tot[q] = red[0][q][lane];
-        for (int w = 1; w < SPMM_WARPS; ++w) {
-          const float4 u = red[w][q][lane];
-          tot[q].x += u.x;
-          tot[q].y += u.y;
-          tot[q].z += u.z;
-          tot[q].w += u.w;
-        }
-      }
-      finish(tot, lrow, ldeg);
-    }
-    __syncthreads();
-  }
+  t->begin[pp->world] = pp->row_begin[pp->world];
+  const int rows = pp->row_begin[pp->rank + 1] - pp->row_begin[pp->rank];
+  CGCN_REQUIRE(rows == n_local, "%s: graph has %d rows, peer block %d", who, n_local, rows);
+  return CGCN_OK;
 }
 
 int spmm_peer_launch(const cgcn_graph* g, const cgcn_peer_panel* pp, float* out, int width, int scale_mode,
                      const float* residual, cudaStream_t stream) {
   CGCN_REQUIRE(g != nullptr && g->rowptr != nullptr && (g->colidx != nullptr || g->nnz == 0), "cgcn_spmm_peer: null graph");
-  CGCN_REQUIRE(pp != nullptr && out != nullptr, "cgcn_spmm_peer: null panel");
-  CGCN_REQUIRE(pp->world >= 1 && pp->world <= CGCN_MAX_PEERS && pp->rank >= 0 && pp->rank < pp->world,
-               "cgcn_spmm_peer: world=%d rank=%d", pp->world, pp->rank);
+  CGCN_REQUIRE(out != nullptr, "cgcn_spmm_peer: null panel");
   CGCN_REQUIRE(g->vals == nullptr, "cgcn_spmm_peer: weighted graphs are not row-partitioned");
   CGCN_REQUIRE(scale_mode == 0 || scale_mode == 1, "cgcn_spmm_peer: scale_mode %d", scale_mode);
   CGCN_REQUIRE(width > 0 && width % 128 == 0 && width <= 1024, "cgcn_spmm_peer: width %d must be a multiple of 128, <= 1024", width);
-  PeerTable t{};
-  t.world = pp->world;
-  for (int r = 0; r < pp->world; ++r) {
-    CGCN_REQUIRE(pp->base[r] != nullptr && pp->row_begin[r] <= pp->row_begin[r + 1], "cgcn_spmm_peer: bad block %d", r);
-    CGCN_REQUIRE(pp->base[r] != out, "cgcn_spmm_peer: in-place aggregation is not possible");
-    t.base[r] = pp->base[r];
-    t.begin[r] = pp->row_begin[r];
-  }
-  t.begin[pp->world] = pp->row_begin[pp->world];
-  CGCN_REQUIRE(pp->row_begin[pp->rank + 1] - pp->row_begin[pp->rank] == g->n, "cgcn_spmm_peer: graph has %d rows, block %d",
-               g->n, pp->row_begin[pp->rank + 1] - pp->row_begin[pp->rank]);
+  PeerTable t;
+  CGCN_TRY(peer_table(&t, pp, g->n, "cgcn_spmm_peer"));
+  for (int r = 0; r < t.world; ++r) CGCN_REQUIRE(t.base[r] != out, "cgcn_spmm_peer: in-place aggregation is not possible");
   if (g->n <= 0) return CGCN_OK;
-  const dim3 grid((g->n + SPMM_WARPS - 1) / SPMM_WARPS), block(SPMM_WARPS * 32);
-#define PEER_CASE(V)                                                                                              \
-  case V:                                                                                                         \
-    spmm_peer_kernel<V><<<grid, block, 0, stream>>>(g->rowptr, g->colidx, g->n, t, out, scale_mode, residual);    \
-    break;
-  switch (width / 128) {
-    PEER_CASE(1)
-    PEER_CASE(2)
-    PEER_CASE(4)
-    PEER_CASE(8)
-    default:
-      set_error("cgcn_spmm_peer: unsupported width %d (128, 256, 512 or 1024)", width);
-      return CGCN_ERR_INVALID;
-  }
-#undef PEER_CASE
-  return check_launch("spmm_peer_kernel");
+  return spmm_run(g, ROWS_PEER, nullptr, t, out, width, scale_mode, residual, stream);
 }
 
 // ---- exchange buffers (CUDA IPC)
@@ -430,32 +328,9 @@ int spmm_launch(const cgcn_graph* g, const float* x, float* out, int width, int 
   CGCN_REQUIRE(scale_mode == 0 || scale_mode == 1, "cgcn_spmm: scale_mode %d", scale_mode);
   CGCN_REQUIRE(width > 0 && width % 128 == 0 && width <= 1024, "cgcn_spmm: width %d must be a multiple of 128, <= 1024", width);
   if (g->n <= 0) return CGCN_OK;
-  const int vec = width / 128;
-  const dim3 grid((g->n + SPMM_WARPS - 1) / SPMM_WARPS), block(SPMM_WARPS * 32);
   const bool weighted = g->vals != nullptr;
   CGCN_REQUIRE(!weighted || g->row_inv != nullptr, "cgcn_spmm: weighted graph without row_inv");
-#define SPMM_CASE(V)                                                                                                  \
-  case V:                                                                                                             \
-    if (weighted)                                                                                                     \
-      CGCN_CUDA(launch_k(spmm_pattern_kernel<V, true>, grid, block, 0, stream, g->rowptr, g->colidx, g->n, x, out,    \
-                         scale_mode, residual, g->vals, g->row_inv));                                                 \
-    else                                                                                                              \
-      CGCN_CUDA(launch_k(spmm_pattern_kernel<V, false>, grid, block, 0, stream, g->rowptr, g->colidx, g->n, x, out,   \
-                         scale_mode, residual, nullptr, nullptr));                                                    \
-    break;
-  switch (vec) {
-    SPMM_CASE(1)
-    SPMM_CASE(2)
-    SPMM_CASE(3)
-    SPMM_CASE(4)
-    SPMM_CASE(6)
-    SPMM_CASE(8)
-    default:
-      set_error("cgcn_spmm: unsupported width %d", width);
-      return CGCN_ERR_INVALID;
-  }
-#undef SPMM_CASE
-  return check_launch("spmm_pattern_kernel");
+  return spmm_run(g, weighted ? ROWS_WEIGHTED : ROWS_PATTERN, x, PeerTable{}, out, width, scale_mode, residual, stream);
 }
 
 }  // namespace cgcn

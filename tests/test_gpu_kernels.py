@@ -45,7 +45,7 @@ def _graph(ip, ix):
     return HiCGraph.from_csr_pattern(ip, ix, _dev(), add_selfloops=True)
 
 
-@pytest.mark.parametrize("width", [128, 256, 512, 1024])
+@pytest.mark.parametrize("width", [128, 256, 384, 512, 768, 1024])
 @pytest.mark.parametrize("mean", [True, False])
 def test_spmm_matches_oracle(width, mean):
     from chromegcn_b200 import ops
@@ -67,12 +67,13 @@ def test_spmm_matches_oracle(width, mean):
     assert ogcn.max_rel(got2, want + res.double()) <= 2e-6
 
 
-@pytest.mark.parametrize("width", [128, 256])
+@pytest.mark.parametrize("width", [128, 256, 512, 1024])
 @pytest.mark.parametrize("n", [1013, 37, 4500])
 def test_spmm_near_diagonal_graph_matches_oracle_and_peer_kernel(width, n):
     """Near-diagonal (Hi-C-like) graphs: short-range pairs, 5 % long-range pairs, one hub row, isolated rows, n not
-    a multiple of the CTA's row count.  Checked against the fp64 oracle and, bit for bit, against the peer-memory
-    kernel with one block (both kernels sum a row's neighbours in CSR order)."""
+    a multiple of the CTA's row count.  Checked against the fp64 oracle and, bit for bit, cgcn_spmm_peer with one
+    block against cgcn_spmm at every width the peer entry point takes: the SpMM kernel reads its rows from the peer
+    table there and from the local panel here, and sums a row's neighbours in CSR order either way."""
     from chromegcn_b200 import ops
     rng = np.random.default_rng(n + width)
     m = n * 8

@@ -67,28 +67,78 @@ def _partitioned(device, rank, world, dropout=0.0, input_grad=True, group=None, 
     return out, loss, {k: p.grad for k, p in m.named_parameters()}, xg, m.batch_norm.running_var, (b, e)
 
 
-@pytest.mark.parametrize("width", [128, 256])
+def _hub_graph(n=3000, hub_row=1500, hub_deg=700):
+    """Near-diagonal pattern of bin(A + I) in which row `hub_row` has `hub_deg` neighbours drawn from all rows."""
+    rng = np.random.default_rng(11)
+    i = rng.integers(0, n, n * 8)
+    j = np.clip(i + rng.integers(-30, 31, n * 8), 0, n - 1)
+    i = np.concatenate([i, np.full(hub_deg, hub_row)])
+    j = np.concatenate([j, rng.choice(n, hub_deg, replace=False)])
+    keep = i != j
+    return oadj.pattern_with_selfloops(*oadj._pairs_to_csr(n, i[keep], j[keep]))
+
+
+@pytest.mark.parametrize("width", [128, 256, 512, 1024])
 @pytest.mark.parametrize("mean", [True, False])
 def test_spmm_peer_blocks_on_one_device_match_spmm(width, mean):
     """The peer-memory SpMM with the panel split into 3 uneven blocks (three separate allocations on one GPU stand
-    in for three ranks' exchange buffers) is bit-identical to the single-panel SpMM on every block's rows."""
+    in for three ranks' exchange buffers) is bit-identical to the single-panel SpMM on every block's rows.  Two graphs:
+    the golden stress graph, and one whose middle block holds a hub row (> LONG_ROW = 512 entries, split over the
+    CTA's warps) with neighbours in all three blocks."""
     from chromegcn_b200 import dist as cdist, ops
     from chromegcn_b200.graph import HiCGraph
     dev = torch.device("cuda", 0)
     z = np.load(os.path.join(GOLDEN, "model_l2_stress.npz"))
-    rp, ci = oadj.pattern_with_selfloops(z["indptr"], z["indices"])
-    n = rp.shape[0] - 1
-    gen = torch.Generator(device=dev).manual_seed(5)
-    x = torch.randn(n, width, device=dev, generator=gen)
-    res = torch.randn(n, width, device=dev, generator=gen)
-    full = ops.spmm(HiCGraph.from_csr_pattern(rp, ci, dev, add_selfloops=False), x, mean=mean, residual=res)
-    cuts = [0, n // 5, n // 5 + n // 2, n]
-    blocks = [x[cuts[r]: cuts[r + 1]].clone() for r in range(3)]
-    for r in range(3):
-        lp, lc = cdist.local_rows_csr(rp, ci, cuts[r], cuts[r + 1])
-        g = HiCGraph.from_csr_pattern(lp, lc, dev, add_selfloops=False)
-        got = ops.spmm_peer(g, blocks, r, mean=mean, residual=res[cuts[r]: cuts[r + 1]])
-        assert torch.equal(got, full[cuts[r]: cuts[r + 1]]), r
+    hub_rp, hub_ci = _hub_graph()
+    hub = hub_ci[hub_rp[1500]: hub_rp[1501]]                   # row 1500 of block [600, 2100)
+    assert hub.shape[0] > 512 and all(((hub >= b) & (hub < e)).any() for b, e in ((0, 600), (600, 2100), (2100, 3000)))
+    for rp, ci in (oadj.pattern_with_selfloops(z["indptr"], z["indices"]), (hub_rp, hub_ci)):
+        n = rp.shape[0] - 1
+        cuts = [0, n // 5, n // 5 + n // 2, n]
+        gen = torch.Generator(device=dev).manual_seed(5)
+        x = torch.randn(n, width, device=dev, generator=gen)
+        res = torch.randn(n, width, device=dev, generator=gen)
+        full = ops.spmm(HiCGraph.from_csr_pattern(rp, ci, dev, add_selfloops=False), x, mean=mean, residual=res)
+        blocks = [x[cuts[r]: cuts[r + 1]].clone() for r in range(3)]
+        for r in range(3):
+            lp, lc = cdist.local_rows_csr(rp, ci, cuts[r], cuts[r + 1])
+            g = HiCGraph.from_csr_pattern(lp, lc, dev, add_selfloops=False)
+            got = ops.spmm_peer(g, blocks, r, mean=mean, residual=res[cuts[r]: cuts[r + 1]])
+            assert torch.equal(got, full[cuts[r]: cuts[r + 1]]), (n, r)
+
+
+def test_spmm_peer_rejects_invalid_panel():
+    """cgcn_spmm_peer checks the peer panel on the host: each malformed panel, an output that is one of the blocks
+    and a width the peer entry point has no kernel for (384) return CGCN_ERR_INVALID before anything is launched."""
+    import ctypes as C
+    from chromegcn_b200 import _lib, dist as cdist, ops
+    from chromegcn_b200.graph import HiCGraph
+    dev = torch.device("cuda", 0)
+    lib = _lib.load()
+    n, cuts = 3000, [0, 600, 2100, 3000]
+    rp, ci = _hub_graph(n)
+    lp, lc = cdist.local_rows_csr(rp, ci, cuts[1], cuts[2])
+    g = HiCGraph.from_csr_pattern(lp, lc, dev, add_selfloops=False)
+    x = {w: torch.randn(n, w, device=dev) for w in (128, 384)}
+    out = {w: torch.empty(g.n, w, device=dev) for w in (128, 384)}
+
+    def call(width=128, world=3, rank=1, begins=cuts, bases=None, o=None):
+        pp = ops.peer_panel([x[width][cuts[r]].data_ptr() for r in range(3)], begins, rank)
+        pp.world = world
+        for r, b in enumerate(bases or []):
+            pp.base[r] = b
+        o = out[width].data_ptr() if o is None else o
+        return lib.cgcn_spmm_peer(C.byref(g.c_struct()), C.byref(pp), o, width, 1, None, _lib.current_stream())
+
+    assert call() == 0                                    # the panel the bad cases below are derived from
+    torch.cuda.synchronize()
+    bad = [dict(world=0), dict(world=9), dict(rank=3), dict(rank=-1), dict(bases=[x[128][0].data_ptr(), None]),
+           dict(begins=[0, 2100, 600, 3000]), dict(begins=[0, 600, 2101, 3000]), dict(o=x[128][cuts[2]].data_ptr()),
+           dict(width=384)]
+    before = _lib.launch_count()
+    for kw in bad:
+        assert call(**kw) == -1, kw                       # CGCN_ERR_INVALID
+    assert _lib.launch_count() == before
 
 
 @pytest.mark.parametrize("exchange", ["nccl", "peer"])
