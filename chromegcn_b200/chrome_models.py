@@ -11,7 +11,7 @@ fp32 and the shared library must be built.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, List, Optional, Tuple
+from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -143,28 +143,52 @@ def fill_params(ps: _lib.Params, tensors: Dict[str, Optional[torch.Tensor]], lay
     ps.out_w, ps.out_b = p("out.weight"), p("out.bias")
 
 
-def build_model_struct(graph: HiCGraph, d: int, nclass: int, layers: int, strands: int, training: bool, dropout_p: float,
-                       seed: int, step: int, params: Dict[str, torch.Tensor], grads: Optional[Dict[str, torch.Tensor]],
-                       running_mean: torch.Tensor, running_var: torch.Tensor, num_batches: Optional[torch.Tensor],
-                       x_in: torch.Tensor, x_in_grad: Optional[torch.Tensor], out: torch.Tensor,
-                       gates: List[Optional[torch.Tensor]], out_grad: Optional[torch.Tensor], workspace: torch.Tensor,
-                       gemm_impl: int = 0, bn_momentum: float = 0.1, bn_eps: float = 1e-5, out_ld: int = 0,
-                       gate_off: bool = False) -> _lib.Model:
+def call_buffers(model: "ChromeGCN", n: int, strands: int, alloc: Callable[[str, int], torch.Tensor],
+                 out_grad: bool = False):
+    """The buffers of one model call over `n` rows: `(workspace, out, out_grad, gates)` -- the workspace
+    `cgcn_model_workspace_bytes` asks for, the logits `[n, strands, padded_classes(nclass)]`, their gradient (None unless
+    `out_grad`) and one `[n, strands]` gate per layer.  `alloc(name, numel)` returns a float32 tensor of at least `numel`
+    elements: a fresh one, or a cached one that is reused from call to call."""
+    d, nclass, layers = model.GC1.in_features, model.out.out_features, model.num_layers
+    ws_bytes = _lib.load().cgcn_model_workspace_bytes(n, d, nclass, layers, strands)
+    if ws_bytes == 0:
+        raise _lib.ChromeGCNNativeError("cgcn_model_workspace_bytes rejected n=%d d=%d" % (n, d))
+    shape = (n, strands, padded_classes(nclass))
+    logits = n * strands * shape[2]
+    ws = alloc("ws", ws_bytes // 4)
+    out = alloc("out", logits)[:logits].view(shape)
+    gates = [alloc("gate%d" % l, n * strands)[: n * strands].view(n, strands) for l in range(layers)]
+    dout = alloc("dout", logits)[:logits].view(shape) if out_grad else None
+    return ws, out, dout, gates
+
+
+def model_struct(model: "ChromeGCN", *, graph: HiCGraph, strands: int, x_in: torch.Tensor,
+                 x_in_grad: Optional[torch.Tensor] = None, params: Dict[str, torch.Tensor],
+                 grads: Optional[Dict[str, torch.Tensor]] = None, out: torch.Tensor, gates: List[torch.Tensor],
+                 out_grad: Optional[torch.Tensor] = None, workspace: torch.Tensor,
+                 dropout_counter: Tuple[int, int]) -> _lib.Model:
+    """The `cgcn_model` struct of one call of `model`.  Everything the module owns comes from it: d, nclass, layers,
+    train / eval mode, dropout rate, `gate_off`, `gemm_impl` and the BatchNorm settings and running statistics.  The
+    caller passes what belongs to the call: graph, strand count, tensors (buffers as `call_buffers` sizes them) and the
+    dropout counter `(seed, step)` the call draws its masks from (`ChromeGCN._next_dropout_counter`)."""
+    layers, bn = model.num_layers, model.batch_norm
+    nclass = model.out.out_features
+    seed, step = dropout_counter
     m = _lib.Model()
-    m.out_ld = out_ld
-    m.gate_off = 1 if gate_off else 0
+    m.out_ld = padded_classes(nclass)
+    m.gate_off = 1 if model.gate_off else 0
     m.graph = graph.c_struct()
-    m.d, m.nclass, m.layers, m.strands = d, nclass, layers, strands
-    m.training = 1 if training else 0
-    m.gemm_impl = gemm_impl
+    m.d, m.nclass, m.layers, m.strands = model.GC1.in_features, nclass, layers, strands
+    m.training = 1 if model.training else 0
+    m.gemm_impl = model.gemm_impl
     m.need_input_grad = 1 if x_in_grad is not None else 0
-    m.dropout_p, m.bn_momentum, m.bn_eps = float(dropout_p), float(bn_momentum), float(bn_eps)
+    m.dropout_p, m.bn_momentum, m.bn_eps = float(model.dropout), bn_momentum(bn), float(bn.eps)
     m.seed, m.step = seed & 0xFFFFFFFFFFFFFFFF, step & 0xFFFFFFFFFFFFFFFF
     fill_params(m.params, params, layers)
     if grads is not None:
         fill_params(m.grads, grads, layers)
-    m.bn_running_mean, m.bn_running_var = _lib.ptr(running_mean), _lib.ptr(running_var)
-    m.bn_num_batches_tracked = _lib.ptr(num_batches)
+    m.bn_running_mean, m.bn_running_var = _lib.ptr(bn.running_mean), _lib.ptr(bn.running_var)
+    m.bn_num_batches_tracked = _lib.ptr(bn.num_batches_tracked)
     m.x_in, m.x_in_grad, m.out = _lib.ptr(x_in), _lib.ptr(x_in_grad), _lib.ptr(out)
     for l in range(layers):
         m.gate[l] = _lib.ptr(gates[l])
@@ -183,53 +207,40 @@ class _ChromeGCNFn(torch.autograd.Function):
         names = module._param_names()
         params = {k: ops._f32c(t.detach()) for k, t in zip(names, param_tensors)}
         x = ops._f32c(x_in.detach())
-        n, d = x.shape
-        nclass, layers = module.out.out_features, module.num_layers
+        n, nclass, layers = x.shape[0], module.out.out_features, module.num_layers
         dev = x.device
-        training = module.training
         with torch.cuda.device(dev):
-            ws_bytes = lib.cgcn_model_workspace_bytes(n, d, nclass, layers, 1)
-            if ws_bytes == 0:
-                raise _lib.ChromeGCNNativeError("cgcn_model_workspace_bytes rejected n=%d d=%d" % (n, d))
-            ws = torch.empty(ws_bytes // 4, dtype=torch.float32, device=dev)
-            ld = padded_classes(nclass)
-            out_buf = torch.empty(n, ld, dtype=torch.float32, device=dev)
-            out = out_buf
-            gates = [torch.empty(n, 1, dtype=torch.float32, device=dev) for _ in range(layers)]
-            seed, step = module._next_dropout_counter() if training else (0, 0)
-            bn = module.batch_norm
-            m = build_model_struct(graph, d, nclass, layers, 1, training, module.dropout, seed, step, params, None,
-                                   bn.running_mean, bn.running_var, bn.num_batches_tracked, x, None, out, gates, None, ws,
-                                   module.gemm_impl, bn_momentum(bn), bn.eps, ld,
-                                   module.gate_off)
+            # fresh buffers: the workspace and the logits are saved for the backward of this node
+            ws, out, _, gates = call_buffers(module, n, 1, lambda name, numel: torch.empty(numel, dtype=torch.float32,
+                                                                                          device=dev))
+            counter = module._next_dropout_counter()
+            m = model_struct(module, graph=graph, strands=1, x_in=x, params=params, out=out, gates=gates, workspace=ws,
+                             dropout_counter=counter)
             _lib.check(lib.cgcn_model_forward(C.byref(m)), "cgcn_model_forward")
         ctx.module, ctx.graph, ctx.names = module, graph, names
-        ctx.cfg = (n, d, nclass, layers, training, seed, step)
-        ctx.save_for_backward(x, ws, out_buf, *gates, *[params[k] for k in names])
+        ctx.training, ctx.counter = module.training, counter
+        ctx.save_for_backward(x, ws, out, *gates, *[params[k] for k in names])
         ctx.mark_non_differentiable(*gates)
-        return (out_buf[:, :nclass], *gates)
+        return (out[:, 0, :nclass], *gates)
 
     @staticmethod
     def backward(ctx, dout, *unused):
         lib = _lib.load()
         module, graph, names = ctx.module, ctx.graph, ctx.names
-        n, d, nclass, layers, training, seed, step = ctx.cfg
+        layers = module.num_layers
         saved = ctx.saved_tensors
         x, ws, out = saved[0], saved[1], saved[2]
         gates = list(saved[3:3 + layers])
         params = dict(zip(names, saved[3 + layers:]))
         dev = x.device
-        ld = out.shape[1]
-        dpad = torch.zeros(n, ld, dtype=torch.float32, device=dev)
-        dpad[:, :nclass] = dout
-        dout = dpad
+        dpad = torch.zeros_like(out)
+        dpad[:, 0, :dout.shape[1]] = dout
         with torch.cuda.device(dev):
             grads = {k: torch.empty_like(v) for k, v in params.items()}
             dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
-            bn = module.batch_norm
-            m = build_model_struct(graph, d, nclass, layers, 1, training, module.dropout, seed, step, params, grads,
-                                   bn.running_mean, bn.running_var, None, x, dx, out, gates, dout, ws, module.gemm_impl,
-                                   bn_momentum(bn), bn.eps, ld, module.gate_off)
+            m = model_struct(module, graph=graph, strands=1, x_in=x, x_in_grad=dx, params=params, grads=grads, out=out,
+                             gates=gates, out_grad=dpad, workspace=ws, dropout_counter=ctx.counter)
+            m.training = 1 if ctx.training else 0            # the mode the forward ran in
             _lib.check(lib.cgcn_model_backward(C.byref(m)), "cgcn_model_backward")
         return (dx, None, None, *[grads[k] for k in names])
 
@@ -257,6 +268,7 @@ class ChromeGCN(nn.Module):
             n_layers = int(layers)
         else:
             n_layers = 2 if layers == 2 else 1
+        self.num_layers = n_layers
         self.GC1 = GraphConvolution(nfeat, nhid, bias=True, init="xavier")
         self.W1 = nn.Linear(nfeat, 1)
         for l in range(2, n_layers + 1):
@@ -272,13 +284,6 @@ class ChromeGCN(nn.Module):
         self._drop_step = 0
 
     # -- helpers shared with the fused trainer
-    @property
-    def num_layers(self) -> int:
-        n = 1
-        while n < MAX_LAYERS and hasattr(self, "GC%d" % (n + 1)):
-            n += 1
-        return n
-
     def _param_names(self) -> List[str]:
         return param_order(self.num_layers)
 
@@ -287,6 +292,10 @@ class ChromeGCN(nn.Module):
         return [sd[k] for k in self._param_names()]
 
     def _next_dropout_counter(self) -> Tuple[int, int]:
+        """`(seed, step)` of the dropout masks of the next forward call: advances once per call in training mode,
+        `(0, 0)` in eval mode (no dropout)."""
+        if not self.training:
+            return 0, 0
         if self._drop_seed is None:
             self._drop_seed = int(torch.randint(0, 2 ** 62, (1,)).item())     # follows torch.manual_seed
         self._drop_step += 1

@@ -48,10 +48,11 @@ def active_in_round(shards: Sequence[Sequence[str]], t: int) -> int:
     return sum(1 for s in shards if t < len(s))
 
 
-def allreduce_gradients(flat_grad: torch.Tensor, group=None) -> None:
-    """The one collective of the chromosome-sharded step: sum of the flat gradient buffer."""
+def allreduce_gradients(t: torch.Tensor, group=None) -> None:
+    """In-place sum over the ranks of `group` of the flat gradient buffer (or, in the row-partitioned step, of the
+    BatchNorm column sums and the loss); nothing without an initialised process group of more than one rank."""
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
-        dist.all_reduce(flat_grad, op=dist.ReduceOp.SUM, group=group)
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
 
 
 class NativeComm:
@@ -166,23 +167,32 @@ def sharded_train_epoch(engine, optimizer, schedule, rank: int, graphs, panels, 
     rank's chromosomes (device resident).  `losses[i]` receives the loss of this rank's i-th chromosome.
     Every round ends with ONE all-reduce of the flat gradient buffer and the same optimiser step on every rank,
     on the mean gradient of the round's chromosomes."""
-    from .engine import flat_params
-    fp = flat_params(engine.model)
     if schedule and isinstance(schedule[0], (list, tuple)) and (not schedule[0] or isinstance(schedule[0][0], str)):
         shards = schedule                                        # per-rank lists: lock-step, one chromosome per cell
         schedule = [[[s[t]] if t < len(s) else [] for s in shards] for t in range(num_rounds(shards))]
-    acc = None
-    i = 0
-    bn = engine.model.batch_norm
+    cells = [rnd[rank] for rnd in schedule]
+    totals = [sum(len(cell) for cell in rnd) for rnd in schedule]
+    for i, c in enumerate(sharded_rounds(engine.model, optimizer, cells, totals, group)):
+        engine.run(graphs[c], panels[c], targets[c], probs[c], losses[i: i + 1], train=True)
+
+
+def sharded_rounds(model, optimizer, cells, totals, group=None):
+    """One rank's chromosome-sharded pass as an iterator: yields the chromosomes of `cells[r]` round by round, and the
+    caller runs each one's train step before it asks for the next.  In between this does the rest of the round: a
+    cell's gradients are summed (every backward overwrites the flat gradient buffer), an empty cell contributes zeros,
+    and the round ends with one all-reduce of the flat gradient buffer and `step_on_mean` over the `totals[r]`
+    chromosomes all ranks ran in round r.  The pass ends with `sync_batchnorm_buffers`."""
+    from .engine import flat_params
+    fp = flat_params(model, full=False)
+    bn = model.batch_norm
     nbt_before = bn.num_batches_tracked.clone() if bn.num_batches_tracked is not None else None
-    for rnd in schedule:
-        mine = rnd[rank]
+    acc = None
+    for mine, total in zip(cells, totals):
         if len(mine) == 0:
             fp.flat_grad.zero_()
         for j, c in enumerate(mine):
-            engine.run(graphs[c], panels[c], targets[c], probs[c], losses[i: i + 1], train=True)
-            i += 1
-            if len(mine) > 1:                                    # accumulate over the cell (backward overwrites)
+            yield c
+            if len(mine) > 1:
                 if j == 0:
                     acc = fp.flat_grad.clone() if acc is None else acc.copy_(fp.flat_grad)
                 else:
@@ -190,8 +200,8 @@ def sharded_train_epoch(engine, optimizer, schedule, rank: int, graphs, panels, 
         if len(mine) > 1:
             fp.flat_grad.copy_(acc)
         allreduce_gradients(fp.flat_grad, group)
-        step_on_mean(optimizer, fp.flat_grad, 1.0 / max(sum(len(cell) for cell in rnd), 1))
-    sync_batchnorm_buffers(engine.model, group, nbt_before)
+        step_on_mean(optimizer, fp.flat_grad, 1.0 / max(total, 1))
+    sync_batchnorm_buffers(model, group, nbt_before)
 
 
 def step_on_mean(optimizer, flat_grad: torch.Tensor, scale: float) -> None:
@@ -385,6 +395,8 @@ class RowPartitionedStep:
             raise ValueError("exchange must be 'nccl' or 'peer'")
         self.exchange = exchange
         self.peer: PeerExchange = None
+        self._x_full: torch.Tensor = None                    # all-gathered panel (nccl exchange)
+        self._bn_sums: torch.Tensor = None                   # BatchNorm column sums, all-reduced
 
     def close(self) -> None:
         if self.peer is not None:
@@ -395,10 +407,6 @@ class RowPartitionedStep:
         w = x_full.shape[1]
         allgather_panel(local_panel.reshape(self.n_local, w), self.parts, out=x_full, group=self.group)
 
-    def _allreduce(self, t: torch.Tensor) -> None:
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size(self.group) > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
-
     def run(self, panel_local: torch.Tensor, target_local: torch.Tensor, loss_out: torch.Tensor, train: bool = True,
             probs_out: torch.Tensor = None, input_grad: torch.Tensor = None):
         """panel_local `[n_local, S, d]`, target_local `[n_local, C]`; returns local logits `[n_local, S, C]`.
@@ -406,35 +414,27 @@ class RowPartitionedStep:
         flat gradient buffer."""
         import ctypes as C
         from . import _lib, ops
-        from .chrome_models import bn_momentum, build_model_struct, padded_classes
+        from .chrome_models import model_struct
         from .engine import flat_params
         lib = _lib.load()
-        model, eng, S = self.model, self.engine, self.S
+        model, S = self.model, self.S
         fp = flat_params(model, full=False)
-        n, d = self.n_local, panel_local.shape[-1]
-        nclass, layers = model.out.out_features, model.num_layers
-        ld = padded_classes(nclass)
+        n, d, nclass, layers = self.n_local, model.GC1.in_features, model.out.out_features, model.num_layers
         dev = panel_local.device
         W = S * d
         with torch.cuda.device(dev):
-            ws_bytes = lib.cgcn_model_workspace_bytes(n, d, nclass, layers, S)
-            ws = eng._buf("ws", ws_bytes // 4)
-            out = eng._buf("out", n * S * ld)[: n * S * ld].view(n, S, ld)
-            dout = eng._buf("dout", n * S * ld)[: n * S * ld].view(n, S, ld)
-            gates = [eng._buf("gate%d" % l, n * S)[: n * S].view(n, S) for l in range(layers)]
+            ws, out, dout, gates = self.engine.call_buffers(n, out_grad=train)
             use_peer = self.exchange == "peer"
             if use_peer and self.peer is None:
                 self.peer = PeerExchange(self.parts, self.rank, W, dev, self.group)
-            x_full = None if use_peer else eng._buf("x_full", self.n_total * W)[: self.n_total * W].view(self.n_total, W)
-            bn_sums = eng._buf("bn_sums", 2 * S * d, dtype=torch.float64)[: 2 * S * d]
-            seed, step = model._next_dropout_counter() if model.training else (0, 0)
-            bn = model.batch_norm
-            m = build_model_struct(self.graph, d, nclass, layers, S, model.training, model.dropout, seed, step,
-                                   fp.views(fp.flat), fp.views(fp.flat_grad) if train else None, bn.running_mean,
-                                   bn.running_var, bn.num_batches_tracked, panel_local, input_grad, out, gates,
-                                   dout if train else None, ws, model.gemm_impl,
-                                   bn_momentum(bn), bn.eps, ld,
-                                   getattr(model, "gate_off", False))
+            if not use_peer and self._x_full is None:
+                self._x_full = torch.empty(self.n_total, W, dtype=torch.float32, device=dev)
+            if self._bn_sums is None:
+                self._bn_sums = torch.empty(2 * S * d, dtype=torch.float64, device=dev)
+            x_full, bn_sums = self._x_full, self._bn_sums
+            m = model_struct(model, graph=self.graph, strands=S, x_in=panel_local, x_in_grad=input_grad,
+                             params=fp.views(fp.flat), grads=fp.views(fp.flat_grad) if train else None, out=out,
+                             gates=gates, out_grad=dout, workspace=ws, dropout_counter=model._next_dropout_counter())
             m.n_total, m.row_begin = self.n_total, self.parts[self.rank][0]
             m.x_full, m.bn_sums = (None if use_peer else x_full.data_ptr()), bn_sums.data_ptr()
             pub = C.c_void_p(0)
@@ -465,27 +465,24 @@ class RowPartitionedStep:
                 if p:
                     gather_ptr(p)
             if model.training:
-                self._allreduce(bn_sums)
+                allreduce_gradients(bn_sums, self.group)
             phase(PHASE_FWD_HEAD)
             loss_local = torch.zeros(1, dtype=torch.float32, device=dev)
-            bce_ws = eng._buf("bce_ws", lib.cgcn_bce_workspace_bytes(n, nclass) // 4 + 64)
-            tgt = ops._f32c(target_local)
-            _lib.check(lib.cgcn_bce_loss(out.data_ptr(), tgt.data_ptr(), n, nclass, S, ld, self.n_total, _lib.ptr(probs_out),
-                                         loss_local.data_ptr(), dout.data_ptr() if train else None, bce_ws.data_ptr(),
-                                         bce_ws.numel() * 4, _lib.current_stream()), "cgcn_bce_loss")
-            self._allreduce(loss_local)
+            ops.bce_loss(out, target_local, S, loss_local, want_probs=False, want_grad=False, n_total=self.n_total,
+                         nclass=nclass, probs_out=probs_out, grad_out=dout, workspace=self.engine.loss_workspace(n))
+            allreduce_gradients(loss_local, self.group)
             loss_out += loss_local
             if not train:
                 return out[:, :, :nclass], gates
             # ---- backward
             phase(PHASE_BWD_HEAD)
-            self._allreduce(bn_sums)
+            allreduce_gradients(bn_sums, self.group)
             for l in range(layers - 1, -1, -1):
                 p = phase(PHASE_BWD_LAYER, l)
                 if p:
                     gather_ptr(p)
             if input_grad is not None:
                 phase(PHASE_BWD_INPUT)
-            self._allreduce(fp.flat_grad)
+            allreduce_gradients(fp.flat_grad, self.group)
             fp.attach_grads()
         return out[:, :, :nclass], gates

@@ -18,7 +18,7 @@ from typing import Dict, List, Optional
 import torch
 
 from . import _lib, ops
-from .chrome_models import ChromeGCN, bn_momentum, build_model_struct, padded_classes
+from .chrome_models import ChromeGCN, call_buffers, model_struct
 from .graph import HiCGraph
 
 _SLOT = 64  # floats: every parameter starts on a 256-byte boundary inside the flat buffer
@@ -130,6 +130,14 @@ class ChromosomeEngine:
         n, d = x_f.shape
         return ops.interleave_strands([x_f, x_r], out=self.panel(n, d))
 
+    def call_buffers(self, n: int, out_grad: bool):
+        """`chrome_models.call_buffers` for a call over `n` rows, served from this engine's cache."""
+        return call_buffers(self.model, n, self.strands, self._buf, out_grad)
+
+    def loss_workspace(self, n: int) -> torch.Tensor:
+        """Workspace of `ops.bce_loss` for `n` rows, served from this engine's cache."""
+        return self._buf("bce_ws", _lib.load().cgcn_bce_workspace_bytes(n, self.model.out.out_features) // 4 + 64)
+
     def run(self, graph: HiCGraph, panel: torch.Tensor, target: torch.Tensor, probs_out: Optional[torch.Tensor],
             loss_slot: torch.Tensor, train: bool, input_grad: Optional[torch.Tensor] = None):
         """One chromosome: forward (+ loss, + backward when `train`).  Gradients land in the model's flat
@@ -138,46 +146,27 @@ class ChromosomeEngine:
         lib = _lib.load()
         model = self.model
         fp = flat_params(model, full=False)
-        S = self.strands
-        n, d = panel.shape[0], panel.shape[-1]
-        nclass, layers = model.out.out_features, model.num_layers
-        dev = panel.device
-        with torch.cuda.device(dev):
-            ws_bytes = lib.cgcn_model_workspace_bytes(n, d, nclass, layers, S)
-            if ws_bytes == 0:
-                raise _lib.ChromeGCNNativeError("cgcn_model_workspace_bytes rejected n=%d d=%d" % (n, d))
-            ws = self._buf("ws", ws_bytes // 4)
-            ld = padded_classes(nclass)
-            out = self._buf("out", n * S * ld)[: n * S * ld].view(n, S, ld)
-            gates = [self._buf("gate%d" % l, n * S)[: n * S].view(n, S) for l in range(layers)]
-            dout = self._buf("dout", n * S * ld)[: n * S * ld].view(n, S, ld)
-            seed, step = model._next_dropout_counter() if model.training else (0, 0)
-            bn = model.batch_norm
-            params = fp.views(fp.flat)
-            grads = fp.views(fp.flat_grad)
-            m = build_model_struct(graph, d, nclass, layers, S, model.training, model.dropout, seed, step, params,
-                                   grads if train else None, bn.running_mean, bn.running_var, bn.num_batches_tracked,
-                                   panel, input_grad, out, gates, None, ws, model.gemm_impl,
-                                   bn_momentum(bn), bn.eps, ld,
-                                   getattr(model, "gate_off", False))
-            bits = target.dtype == torch.int32            # ops.pack_targets bit rows
-            if bits:
-                if target.shape != (n, (nclass + 31) // 32):
-                    raise ValueError("bit-packed targets must be [n, ceil(nclass/32)] int32")
-                tgt = target.contiguous()
-            else:
-                tgt = ops._f32c(target)
+        n, nclass = panel.shape[0], model.out.out_features
+        with torch.cuda.device(panel.device):
+            ws, out, dout, gates = self.call_buffers(n, out_grad=train)
+            m = model_struct(model, graph=graph, strands=self.strands, x_in=panel, x_in_grad=input_grad,
+                             params=fp.views(fp.flat), grads=fp.views(fp.flat_grad) if train else None, out=out,
+                             gates=gates, workspace=ws, dropout_counter=model._next_dropout_counter())
             if train:
+                bits = target.dtype == torch.int32            # ops.pack_targets bit rows
+                if bits:
+                    if target.shape != (n, (nclass + 31) // 32):
+                        raise ValueError("bit-packed targets must be [n, ceil(nclass/32)] int32")
+                    tgt = target.contiguous()
+                else:
+                    tgt = ops._f32c(target)
                 step_fn = lib.cgcn_train_step_bits if bits else lib.cgcn_train_step
                 _lib.check(step_fn(C.byref(m), tgt.data_ptr(), _lib.ptr(probs_out), loss_slot.data_ptr(),
                                    dout.data_ptr()), "cgcn_train_step")
                 fp.attach_grads()
             else:
                 _lib.check(lib.cgcn_model_forward(C.byref(m)), "cgcn_model_forward")
-                bce_ws = self._buf("bce_ws", lib.cgcn_bce_workspace_bytes(n, nclass) // 4 + 64)
-                loss_fn = lib.cgcn_bce_loss_bits if bits else lib.cgcn_bce_loss
-                _lib.check(loss_fn(out.data_ptr(), tgt.data_ptr(), n, nclass, S, ld, 0, _lib.ptr(probs_out),
-                                   loss_slot.data_ptr(), None, bce_ws.data_ptr(), bce_ws.numel() * 4,
-                                   _lib.current_stream()), "cgcn_bce_loss")
+                ops.bce_loss(out, target, self.strands, loss_slot, want_probs=False, want_grad=False, nclass=nclass,
+                             probs_out=probs_out, workspace=self.loss_workspace(n))
         self.step_count += 1
         return out[:, :, :nclass], gates

@@ -173,17 +173,14 @@ def finetune(WindowModel, ChromeModel, chrom_feature_dict, crit, optimizer, epoc
     chroms = list(chrom_feature_dict.keys())
     # Chromosome-sharded pass (one process per GPU, SURVEY.md 8(e)): `opt.shard = (schedule, rank, group)` with
     # `schedule[round][rank]` = chromosomes (dist.balanced_schedule).  This rank streams only ITS chromosomes, in
-    # schedule order; gradients accumulate over a round's cell, every round ends with one all-reduce of the flat
-    # gradient buffer and the same optimiser step on every rank (mean gradient of the round's chromosomes).
+    # schedule order; in training `dist.sharded_rounds` accumulates the gradients over a round's cell and ends every
+    # round with one all-reduce of the flat gradient buffer and the same optimiser step on every rank (mean gradient
+    # of the round's chromosomes).
     shard = getattr(opt, "shard", None)
     if shard is not None:
         schedule, shard_rank, shard_group = shard
-        rounds = [[c for c in rnd[shard_rank] if c in chrom_feature_dict] for rnd in schedule]
-        round_totals = [max(sum(len(cell) for cell in rnd), 1) for rnd in schedule]
-        chroms = [c for r in rounds for c in r]
-    else:
-        rounds = [[c] for c in chroms]
-        round_totals = [1] * len(rounds)
+        cells = [[c for c in rnd[shard_rank] if c in chrom_feature_dict] for rnd in schedule]
+        chroms = [c for cell in cells for c in cell]
     sizes = {c: chrom_feature_dict[c]["forward"].size(0) for c in chroms}
     nclass = ChromeModel.out.out_features
     graphs = graphs_for(opt, split, chroms, sizes, device)
@@ -244,57 +241,39 @@ def finetune(WindowModel, ChromeModel, chrom_feature_dict, crit, optimizer, epoc
         if chroms:
             stage(0)
         row = 0
-        k = 0
-        fp = flat_params(ChromeModel, full=False)
-        bn = ChromeModel.batch_norm
-        nbt_before = bn.num_batches_tracked.clone() if (shard is not None and train and bn.num_batches_tracked is not None) else None
-        acc = None
-        for r_idx, mine in enumerate(rounds):
-            for j, chrom in enumerate(mine):
-                if k + 1 < len(chroms):
-                    stage(k + 1)
-                item = staged[k % 2]
-                n = sizes[chrom]
-                if item[0] == "resident":
-                    panel, tgt = item[1], item[2]
-                else:
-                    main.wait_event(ready[k % 2])
-                    _, x_f, x_r, tgt = item
-                    if resident:
-                        panel = ops.interleave_strands([x_f, x_r])
-                        tgt = tgt.clone()
-                        _RESIDENT[(id(chrom_feature_dict), chrom, str(device))] = (
-                            _feature_signature(chrom_feature_dict[chrom]), panel, tgt)
-                    else:
-                        panel = engine.pack(x_f, x_r)
-                if train and shard is None:
-                    optimizer.zero_grad()                                    # finetune.py:39
-                engine.run(graphs[chrom], panel, tgt, all_preds_dev[row: row + n], losses_dev[k: k + 1], train)
-                if train and shard is None:
-                    optimizer.step()                                         # finetune.py:49
-                elif train and len(mine) > 1:                                # accumulate over the cell (backward overwrites)
-                    if j == 0:
-                        acc = fp.flat_grad.clone() if acc is None else acc.copy_(fp.flat_grad)
-                    else:
-                        acc.add_(fp.flat_grad)
-                consumed[k % 2].record(main)
-                # predictions of this chromosome go home while the next one computes (finetune.py:52)
-                d2h.wait_event(consumed[k % 2])
-                with torch.cuda.stream(d2h):
-                    all_preds[row: row + n].copy_(all_preds_dev[row: row + n], non_blocking=True)
-                row += n
-                k += 1
-            if train and shard is not None:                                  # end of the round: one collective, one step
-                from . import dist as cdist
-                if len(mine) == 0:
-                    fp.flat_grad.zero_()
-                elif len(mine) > 1:
-                    fp.flat_grad.copy_(acc)
-                cdist.allreduce_gradients(fp.flat_grad, shard_group)
-                cdist.step_on_mean(optimizer, fp.flat_grad, 1.0 / round_totals[r_idx])
+        order = chroms
         if train and shard is not None:
             from . import dist as cdist
-            cdist.sync_batchnorm_buffers(ChromeModel, shard_group, nbt_before)
+            totals = [sum(len(cell) for cell in rnd) for rnd in schedule]
+            order = cdist.sharded_rounds(ChromeModel, optimizer, cells, totals, shard_group)
+        for k, chrom in enumerate(order):
+            if k + 1 < len(chroms):
+                stage(k + 1)
+            item = staged[k % 2]
+            n = sizes[chrom]
+            if item[0] == "resident":
+                panel, tgt = item[1], item[2]
+            else:
+                main.wait_event(ready[k % 2])
+                _, x_f, x_r, tgt = item
+                if resident:
+                    panel = ops.interleave_strands([x_f, x_r])
+                    tgt = tgt.clone()
+                    _RESIDENT[(id(chrom_feature_dict), chrom, str(device))] = (
+                        _feature_signature(chrom_feature_dict[chrom]), panel, tgt)
+                else:
+                    panel = engine.pack(x_f, x_r)
+            if train and shard is None:
+                optimizer.zero_grad()                                    # finetune.py:39
+            engine.run(graphs[chrom], panel, tgt, all_preds_dev[row: row + n], losses_dev[k: k + 1], train)
+            if train and shard is None:
+                optimizer.step()                                         # finetune.py:49
+            consumed[k % 2].record(main)
+            # predictions of this chromosome go home while the next one computes (finetune.py:52)
+            d2h.wait_event(consumed[k % 2])
+            with torch.cuda.stream(d2h):
+                all_preds[row: row + n].copy_(all_preds_dev[row: row + n], non_blocking=True)
+            row += n
         done.record(d2h)
         losses = losses_dev.cpu()                                            # the one sync of the split
         done.synchronize()

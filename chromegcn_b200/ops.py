@@ -80,14 +80,14 @@ def spmm_peer(graph: HiCGraph, blocks: Sequence[torch.Tensor], rank: int, mean: 
     return out
 
 
-def _out(t: Optional[torch.Tensor], shape, device, more_rows: bool = False) -> torch.Tensor:
+def _out(t: Optional[torch.Tensor], shape, device, more_rows: bool = False, align: int = 16) -> torch.Tensor:
     """Output buffer of a kernel: a new tensor, or the caller's, which the kernel writes in place (so it is checked, not
     copied like `_f32c` inputs; a view into a larger buffer is fine).  `more_rows`: the caller's tensor may have more
-    rows than `shape` (per-CTA partials)."""
+    rows than `shape` (per-CTA partials).  `align`: the byte alignment the kernel's stores need."""
     if t is None:
         return torch.empty(*shape, dtype=torch.float32, device=device)
-    if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.data_ptr() % 16 != 0:
-        raise _lib.ChromeGCNNativeError("output tensors must be contiguous, 16-byte aligned CUDA float32")
+    if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.data_ptr() % align != 0:
+        raise _lib.ChromeGCNNativeError("output tensors must be contiguous, %d-byte aligned CUDA float32" % align)
     rows_ok = t.shape[0] >= shape[0] if more_rows else t.shape[0] == shape[0]
     if t.dim() != len(shape) or tuple(t.shape[1:]) != tuple(shape[1:]) or not rows_ok:
         raise _lib.ChromeGCNNativeError("output tensor of shape %s, need %s" % (tuple(t.shape), tuple(shape)))
@@ -235,36 +235,39 @@ def pack_targets(target: torch.Tensor, pin: bool = False) -> Optional[torch.Tens
 
 
 def bce_loss(out: torch.Tensor, target: torch.Tensor, strands: int, loss_acc: torch.Tensor,
-             want_probs: bool = True, want_grad: bool = True, n_total: int = 0, nclass: Optional[int] = None):
-    """finetune.py:43-45,52 on `[n, strands, C]` logits: returns `(probs [n, C] | None, out_grad | None)`
-    and adds the mean loss to `loss_acc[0]`.  An int32 `target` is a `pack_targets` bit matrix (pass `nclass`)."""
+             want_probs: bool = True, want_grad: bool = True, n_total: int = 0, nclass: Optional[int] = None,
+             probs_out: Optional[torch.Tensor] = None, grad_out: Optional[torch.Tensor] = None,
+             workspace: Optional[torch.Tensor] = None):
+    """finetune.py:43-45,52 on `[n, strands, ld]` logits (row pitch ld >= C): returns `(probs [n, C] | None,
+    out_grad | None)` and adds the mean loss to `loss_acc[0]` (over `n_total` rows when the logits are one row block
+    of a larger graph).  An int32 `target` is a `pack_targets` bit matrix (pass `nclass`).  `probs_out` / `grad_out`,
+    when given, receive the results (`want_*` then does not matter); `workspace` is at least
+    `cgcn_bce_workspace_bytes` long."""
     lib = _lib.load()
     out = _f32c(out)
-    ld = out.shape[-1]                       # row pitch of the logits (>= nclass)
-    if target.dtype == torch.int32:
-        if nclass is None or target.shape[1] != (nclass + 31) // 32:
+    dev = out.device
+    bits = target.dtype == torch.int32
+    if bits:
+        if nclass is None or target.dim() != 2 or target.shape[1] != (nclass + 31) // 32:
             raise ValueError("bit-packed targets need nclass with ceil(nclass/32) == target.shape[1]")
-        target = target.contiguous()
-        n, c = target.shape[0], int(nclass)
-        probs = torch.empty(n, c, dtype=torch.float32, device=out.device) if want_probs else None
-        grad = torch.empty_like(out) if want_grad else None
-        with torch.cuda.device(out.device):
-            need = lib.cgcn_bce_workspace_bytes(n, c)
-            ws = torch.empty(need, dtype=torch.uint8, device=out.device)
-            _lib.check(lib.cgcn_bce_loss_bits(out.data_ptr(), target.data_ptr(), n, c, strands, ld, n_total, _lib.ptr(probs),
-                                              loss_acc.data_ptr(), _lib.ptr(grad), ws.data_ptr(), need,
-                                              _lib.current_stream()), "cgcn_bce_loss_bits")
-        return probs, grad
-    target = _f32c(target)
-    n, c = target.shape
-    probs = torch.empty(n, c, dtype=torch.float32, device=out.device) if want_probs else None
-    grad = torch.empty_like(out) if want_grad else None
-    with torch.cuda.device(out.device):
-        need = lib.cgcn_bce_workspace_bytes(n, c)
-        ws = torch.empty(need, dtype=torch.uint8, device=out.device)
-        _lib.check(lib.cgcn_bce_loss(out.data_ptr(), target.data_ptr(), n, c, strands, ld, n_total, _lib.ptr(probs),
-                                     loss_acc.data_ptr(), _lib.ptr(grad), ws.data_ptr(), need, _lib.current_stream()),
-                   "cgcn_bce_loss")
+        target, c = target.contiguous(), int(nclass)
+    else:
+        target = _f32c(target)
+        c = target.shape[1]
+        if nclass is not None and c != nclass:
+            raise ValueError("targets have %d columns, nclass is %d" % (c, nclass))
+    n = target.shape[0]
+    if out.shape[0] != n:
+        raise ValueError("%d logit rows, %d target rows" % (out.shape[0], n))
+    probs = _out(probs_out, (n, c), dev, align=4) if (probs_out is not None or want_probs) else None
+    grad = _out(grad_out, tuple(out.shape), dev) if (grad_out is not None or want_grad) else None
+    with torch.cuda.device(dev):
+        if workspace is None:
+            workspace = torch.empty(lib.cgcn_bce_workspace_bytes(n, c), dtype=torch.uint8, device=dev)
+        name = "cgcn_bce_loss_bits" if bits else "cgcn_bce_loss"
+        _lib.check(getattr(lib, name)(out.data_ptr(), target.data_ptr(), n, c, strands, out.shape[-1], n_total,
+                                      _lib.ptr(probs), loss_acc.data_ptr(), _lib.ptr(grad), _lib.ptr(workspace),
+                                      workspace.numel() * workspace.element_size(), _lib.current_stream()), name)
     return probs, grad
 
 

@@ -586,6 +586,68 @@ def test_sharded_epoch_round_is_one_step_on_the_mean_gradient():
         assert ogcn.max_rel(p.detach().cpu(), q.detach()) <= 2e-5, k
 
 
+def test_finetune_shard_matches_sharded_epoch(tmp_path):
+    """finetune() with `opt.shard` (pinned host features streamed H2D, bit-packed labels) and sharded_train_epoch
+    (device-resident panels, float labels) run the same rounds: from the same weights over the same chromosomes they
+    must end bit-identical -- parameters, BatchNorm running statistics, num_batches_tracked, per-chromosome losses and
+    probabilities.  Rank 0 of a two-rank schedule: round 1 has a two-chromosome cell, round 2 an empty one, and the
+    other rank's chromosomes count in every round's mean."""
+    import argparse
+    import pickle
+    from scipy import sparse
+    from chromegcn_b200 import finetune as ft, ops, synthetic
+    from chromegcn_b200 import dist as cdist
+    from chromegcn_b200.chrome_models import ChromeGCN
+    from chromegcn_b200.engine import ChromosomeEngine
+    from chromegcn_b200.optim import FlatSGD
+    nclass, mine = 9, ["chr20", "chr22", "chr21"]
+    schedule = [[["chr20", "chr22"], ["chr19"]], [[], ["chr18"]], [["chr21"], []]]
+    feats, adj = {}, {}
+    for i, c in enumerate(mine):
+        h = synthetic.make_hic(c, hic_edges=3000, n_windows=300 + 40 * i, n_bins=900)
+        ip, ix = oadj.build_adjacency_numpy(h.window_starts, h.bin1, h.bin2, h.val, h.norm, 1, 3000)
+        n = ip.shape[0] - 1
+        adj[c] = sparse.csr_matrix((np.ones(ix.shape[0]), ix, ip), shape=(n, n))
+        feats[c] = synthetic.make_features(c, n, 128, nclass)
+    with open(tmp_path / "train_graphs_3000_SQRTVCnorm.pkl", "wb") as fp:
+        pickle.dump(adj, fp)
+    opt = argparse.Namespace(adj_type="hic", graph_root=str(tmp_path), hicsize="3000", hicnorm="SQRTVC",
+                             shard=(schedule, 0, None))
+    torch.manual_seed(2)
+    start = ChromeGCN(128, 128, nclass, 0.0, True, 2).state_dict()
+    models = []
+    for _ in range(2):
+        m = ChromeGCN(128, 128, nclass, 0.0, True, 2)
+        m.load_state_dict(start)
+        models.append(m.to(_dev()).train())
+    ft.clear_caches()
+    # finetune() keeps its per-chromosome losses on the device: record each loss slot as its engine returns
+    eng = ft.engine_for(models[0])
+    run, ft_losses = eng.run, []
+
+    def recording_run(graph, panel, target, probs_out, loss_slot, train):
+        res = run(graph, panel, target, probs_out, loss_slot, train)
+        ft_losses.append(loss_slot.clone())
+        return res
+    eng.run = recording_run
+    ft_probs, _, ft_total = ft.finetune(None, models[0], feats, None, FlatSGD(models[0], lr=0.25), 1, None, opt, "train")
+    assert len(ft_losses) == len(mine)
+    graphs = ft.graphs_for(opt, "train", mine, {c: feats[c]["forward"].shape[0] for c in mine}, _dev())
+    panels = {c: ops.interleave_strands([feats[c]["forward"].to(_dev()), feats[c]["backward"].to(_dev())]) for c in mine}
+    targets = {c: feats[c]["target"].to(_dev()) for c in mine}
+    probs = {c: torch.empty(feats[c]["target"].shape, device=_dev()) for c in mine}
+    losses = torch.zeros(len(mine), device=_dev())
+    cdist.sharded_train_epoch(ChromosomeEngine(models[1], 2), FlatSGD(models[1], lr=0.25), schedule, 0, graphs, panels,
+                              targets, probs, losses)
+    assert torch.equal(torch.cat(ft_losses).cpu(), losses.cpu())
+    assert ft_total == float(losses.cpu().double().sum())
+    assert torch.equal(ft_probs, torch.cat([probs[c] for c in mine]).cpu())
+    sd0, sd1 = models[0].state_dict(), models[1].state_dict()
+    assert int(sd1["batch_norm.num_batches_tracked"]) > int(start["batch_norm.num_batches_tracked"])
+    for k in sd0:
+        assert torch.equal(sd0[k].cpu(), sd1[k].cpu()), k
+
+
 def test_module_api_training_loop_with_flat_optimizer_matches_oracle():
     """The reference's own loop -- optimizer.zero_grad(); forward x2 through the module API; loss.backward();
     optimizer.step() (finetune.py:39-49) -- for several steps with this package's ChromeGCN and get_optimizer().  After the
